@@ -238,9 +238,11 @@ int scb_getrf_piv(int64_t n_pad, double* M, double* dinv, int32_t* piv, int32_t*
                   scb_stream_t stream);
 
 /* Solves M X = B in place for nrhs right-hand sides, B[n_pad, nrhs] row-major, with the factors
- * and the `dinv` buffer produced by scb_getrf_nopiv / scb_getrf_sym_nopiv.  One right-hand side: two
- * persistent flag-driven sweep kernels; 2..16: the same sweeps with DMMA block products (8 columns per
- * pass); more: blocked right-looking substitution on DMMA (one launch per 128-row block step). */
+ * and the `dinv` buffer produced by scb_getrf_nopiv / scb_getrf_sym_nopiv / scb_getrf_piv (for the
+ * latter, B holds the permuted right-hand side).  Two persistent flag-driven sweep kernels (forward,
+ * backward) over column chains: one right-hand side: one scalar chain; 2..8: one chain of 8 columns with
+ * DMMA block products; more: chains of 16 columns, at most 8 chains (128 columns) per launch -- beyond
+ * that a further launch pair per 128 columns. */
 int scb_getrs_nopiv(int64_t n_pad, const double* LU, const double* dinv, int64_t nrhs, double* B,
                     scb_stream_t stream);
 

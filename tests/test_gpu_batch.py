@@ -157,8 +157,8 @@ def test_find_fluxoid_solution(sc):
 
 @pytest.mark.parametrize("nrhs", [3, 9, 16, 21, 70])
 def test_many_rhs_tensor_core_substitution(sc, nrhs):
-    """2..16 right-hand sides take the flag-driven DMMA sweeps (getrs.cu: trsv_sweep_dmma_kernel, 8
-    columns per pass), more the blocked DMMA substitution (trsm_rhs_step_kernel); both must agree with
+    """2..8 right-hand sides take the flag-driven DMMA sweeps in one chain of 8 columns (getrs.cu:
+    trsm_sweep_dmma_kernel<8>), more run chains of 16 columns (trsm_sweep_dmma_kernel<16>); both must agree with
     column-by-column solves, including column counts that are not a multiple of the 8- / 16-column
     chunks and a padded last block."""
     import torch
