@@ -293,12 +293,14 @@ enum scb_bs_kind {
   /* solution.py:917-928 vector potential: tgt [m,3], src [n,3], out [m,2] */
   SCB_BS_VECTOR_POTENTIAL = 3,
   /* solve_film.py:393-412 _get_boundary_effective_field: tgt [m,2], src = edge centres [n,2],
-   * J = edge normals [n,2], area = stream * length [n], out [m] */
+   * J = edge normals [n,2], area = stream * length [n, nsets], out [m, nsets].  The edge geometry
+   * (centres, normals, r^-3 of every pair) is shared by the nsets stream sets. */
   SCB_BS_BOUNDARY = 4
 };
 
 /* out = prefactor * sum_j area_j * kernel(tgt_i, src_j, J_j).  nsets > 1 evaluates `nsets`
- * current-density sets J[nsets, n, 2] against the same geometry, out[nsets, m(, c)]. */
+ * current-density sets J[nsets, n, 2] against the same geometry, out[nsets, m(, c)]; for
+ * SCB_BS_BOUNDARY the sets are the columns of area[n, nsets] and out[m, nsets] (see above). */
 int scb_biot_savart(int kind, int64_t m, const double* tgt, int64_t n, const double* src,
                     const double* area, const double* J, double dz, double prefactor,
                     int64_t nsets, double* out, scb_stream_t stream);
@@ -313,6 +315,19 @@ int scb_biot_savart(int kind, int64_t m, const double* tgt, int64_t n, const dou
 int scb_film_coupling(int64_t m, const double* tgt, double tgt_z, int64_t n, const double* src,
                       const double* area, const double* J, int64_t skip_lo, int64_t skip_hi,
                       double prefactor, int64_t nsets, double* out, scb_stream_t stream);
+
+/* Field of a film's own sheet current at its vertices for `nsets` current-density sets
+ * (solve_film.py:415-437 _biot_savart_within_film; the self field of a film with transport terminals):
+ *   out[i, s] = prefactor * sum_j area_j (Jx[j,s] (y_i - y_j) - Jy[j,s] (x_i - x_j)) r_ij^-3,
+ * tgt [m,2] (vertices), src [n,2] (triangle centroids), area [n], J [n, nsets, 2] (source-major: the
+ * layout scb_spmv produces for the triangle gradients), out [m, nsets].  Every full pass of 64 sets runs
+ * as a GEMM on the fp64 tensor cores (K = 2 n) whose r^-3 operand is evaluated in the mma fragment
+ * layout and shared by the 64 sets; the remaining sets run as tiled N-body sums on the CUDA cores in
+ * passes of 8 / 4 / 2 / 1 (faster below 32 sets, even at 32, measured).  Fixed summation order:
+ * bit-reproducible.  n = 0 writes zeros; m = 0 does nothing. */
+int scb_biot_savart_within_film(int64_t m, const double* tgt, int64_t n, const double* src,
+                                const double* area, const double* J, double prefactor, int64_t nsets,
+                                double* out, scb_stream_t stream);
 
 /* ------------------------------------------------------------------------------------
  * Pairwise distances (K20): distance.py:5-84 cdist / (sq)euclidean_distance_2d/3d

@@ -25,7 +25,7 @@ def _nvcc() -> str:
 
 
 STAMP = LIB + ".stamp"
-ABI_VERSION = 201  # must equal scb_version() of the sources (csrc/api.cu)
+ABI_VERSION = 202  # must equal scb_version() of the sources (csrc/api.cu)
 
 
 def source_digest() -> str:

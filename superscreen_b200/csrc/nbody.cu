@@ -41,14 +41,15 @@ struct NbodyParams {
   int64_t n;              // sources
   const double* src;      // [*,2] or [*,3] (indexed through src_idx when given)
   const int64_t* src_idx; // optional gather list for NB_KERNEL
-  const double* area;     // [*] per-source weight
+  const double* area;     // [*] per-source weight; NB_BOUNDARY: [n, ldv] per-source, per-set strengths
   const double* J;        // [*,2] (biot-savart), v [*, ldv] (NB_KERNEL), [n, ldv] (NB_COUPLING, ldv = 2 nsets)
-  int64_t ldv;            // row stride of v / J
-  int64_t ldo;            // row stride of out (NB_KERNEL: = ldv; NB_COUPLING: nsets)
+  int64_t ldv;            // row stride of v / J (NB_BOUNDARY: of area, = nsets)
+  int64_t ldo;            // row stride of out (NB_KERNEL: = ldv; NB_COUPLING, NB_BOUNDARY: nsets)
   int64_t rhs0;           // first rhs column / current-density set handled by this launch
   double dz2;             // film-to-film: squared layer distance
   double tgt_z;           // NB_COUPLING: z of the target film
   int64_t skip_lo, skip_len;  // NB_COUPLING: sources [skip_lo, skip_lo + skip_len) are left out
+  int64_t sld;            // NB_COUPLING: source row (x, y, z) = 3, or (x, y) = 2 for sources in the target plane
   double prefactor;
   double* out;
   int accumulate;
@@ -59,8 +60,10 @@ struct NbodyParams {
 template <int KIND, int NR>
 struct Traits {
   static constexpr int tdim = (KIND == NB_Z || KIND == NB_VECTOR || KIND == NB_VECPOT) ? 3 : 2;
-  // NR = right-hand sides (NB_KERNEL) or current-density sets sharing the geometry (film-to-film)
-  static constexpr bool multi = KIND == NB_KERNEL || KIND == NB_FILM_TO_FILM || KIND == NB_COUPLING;
+  // NR = right-hand sides (NB_KERNEL), current-density sets sharing the geometry (film-to-film) or
+  // boundary stream sets sharing the edges (NB_BOUNDARY)
+  static constexpr bool multi = KIND == NB_KERNEL || KIND == NB_FILM_TO_FILM || KIND == NB_COUPLING ||
+                                KIND == NB_BOUNDARY;
   static constexpr int nacc = multi ? NR : (KIND == NB_VECTOR ? 4 : (KIND == NB_VECPOT || KIND == NB_Z ? 2 : 1));
   static constexpr int npay = KIND == NB_KERNEL ? NR : (multi ? 2 * NR : 2);
   static constexpr bool has_sz = tdim == 3 || KIND == NB_COUPLING;
@@ -76,7 +79,7 @@ __device__ __forceinline__ void nbody_store(const NbodyParams& p, int64_t i, con
       double* o = p.out + i * p.ldo + p.rhs0 + r;
       *o = p.accumulate ? *o + pf * acc[r] : pf * acc[r];
     }
-  } else if (KIND == NB_COUPLING) {
+  } else if (KIND == NB_COUPLING || KIND == NB_BOUNDARY) {
 #pragma unroll
     for (int r = 0; r < NR; r++) p.out[i * p.ldo + p.rhs0 + r] = pf * acc[r];
   } else if (KIND == NB_Z) {
@@ -91,8 +94,6 @@ __device__ __forceinline__ void nbody_store(const NbodyParams& p, int64_t i, con
   } else if (KIND == NB_FILM_TO_FILM) {
 #pragma unroll
     for (int r = 0; r < NR; r++) p.out[r * p.m + i] = pf * acc[r];
-  } else {
-    p.out[i] = pf * acc[0];
   }
 }
 
@@ -134,9 +135,9 @@ __global__ void __launch_bounds__(256) nbody_kernel(NbodyParams p) {
       const int64_t js = p.src_idx ? p.src_idx[j] : j;
       const double w = p.area[js];
       if (KIND == NB_COUPLING) {
-        sx[tid] = p.src[3 * js];
-        sy[tid] = p.src[3 * js + 1];
-        const double dz = p.tgt_z - p.src[3 * js + 2];
+        sx[tid] = p.src[p.sld * js];
+        sy[tid] = p.src[p.sld * js + 1];
+        const double dz = p.tgt_z - (p.sld == 3 ? p.src[3 * js + 2] : p.tgt_z);
         sz[tid] = dz * dz;
         const double* Jj = p.J + js * p.ldv + 2 * p.rhs0;
 #pragma unroll
@@ -156,6 +157,13 @@ __global__ void __launch_bounds__(256) nbody_kernel(NbodyParams p) {
           for (int r = 0; r < NR; r++) {
             spay[2 * r][tid] = w * p.J[(r * p.n + js) * 2];
             spay[2 * r + 1][tid] = w * p.J[(r * p.n + js) * 2 + 1];
+          }
+        } else if (KIND == NB_BOUNDARY) {
+#pragma unroll
+          for (int r = 0; r < NR; r++) {
+            const double wr = p.area[js * p.ldv + p.rhs0 + r];
+            spay[2 * r][tid] = wr * p.J[2 * js];
+            spay[2 * r + 1][tid] = wr * p.J[2 * js + 1];
           }
         } else {
           spay[0][tid] = w * p.J[2 * js];
@@ -200,7 +208,8 @@ __global__ void __launch_bounds__(256) nbody_kernel(NbodyParams p) {
 #pragma unroll
             for (int r = 0; r < NR; r++) acc[k][r] = fma(pay[2 * r], kdy, fma(-pay[2 * r + 1], kdx, acc[k][r]));
           } else if (KIND == NB_BOUNDARY) {
-            acc[k][0] = fma(-k3, fma(pay[0], dx, pay[1] * dy), acc[k][0]);
+#pragma unroll
+            for (int r = 0; r < NR; r++) acc[k][r] = fma(-k3, fma(pay[2 * r], dx, pay[2 * r + 1] * dy), acc[k][r]);
           } else if (KIND == NB_Z) {
             acc[k][0] = fma(k3 * pay[0], dy, acc[k][0]);  // Jx_dy
             acc[k][1] = fma(k3 * pay[1], dx, acc[k][1]);  // Jy_dx
@@ -408,6 +417,105 @@ static int launch_kernel_gemm(const NbodyParams& p, cudaStream_t s) {
   return SCB_OK;
 }
 
+// ---------------------------------------------------------------------------------------
+// Within-film field of many current-density sets (solve_film.py:415-437) on the fp64 tensor cores:
+//   out[i, s] = sum_j a_j (Jx[j,s] dy - Jy[j,s] dx) r_ij^-3   as a GEMM with K = 2 n_src,
+//   A[i, 2j] = dy r^-3,  A[i, 2j+1] = -dx r^-3  (dx = x_i - x_j),   P[2j + c, s] = a_j J[j, s, c].
+// A is evaluated in the mma.sync m8n8k4 A-fragment layout and never stored.  A k-step covers two
+// sources (lanes t = 0, 1: source 0, components x, y; t = 2, 3: source 1), so a group of four sources
+// spans two k-steps: lane (g, t) evaluates r^-3 of target g and source t of the group once, and each
+// k-step fetches the (source, component) entry its fragment needs from lane (g, 2h + t/2) by shuffle.
+// One r^-3 then serves NC = 8 CT sets.  CTA: 64 targets (8 warps x 8 rows); sources in tiles of 16
+// (32 k rows), double-buffered through registers as in kernel_gemm_kernel.  Every output is summed
+// by one lane in a fixed order: no atomics, bit-reproducible.
+// ---------------------------------------------------------------------------------------
+constexpr int kWfSrc = 16;
+
+template <int CT>
+__global__ void __launch_bounds__(256, 2) within_film_gemm_kernel(NbodyParams p) {
+  constexpr int NC = 8 * CT;
+  constexpr int KR = 2 * kWfSrc;                 // k rows of a source tile
+  constexpr int PLD = NC + 4;                    // conflict-free B fragments (ld % 16 == 4)
+  constexpr int PER = KR * NC / 256;             // payload entries staged per thread
+  __shared__ double sx[2][kWfSrc], sy[2][kWfSrc];
+  __shared__ double sp[2][KR * PLD];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int g = lane >> 2, t = lane & 3;
+  const int64_t i = blockIdx.x * 64ll + warp * 8 + g;
+  const bool active = i < p.m;
+  const double tx = active ? p.tgt[2 * i] : 0.0, ty = active ? p.tgt[2 * i + 1] : 0.0;
+  double acc[CT][2];
+#pragma unroll
+  for (int c = 0; c < CT; c++) acc[c][0] = acc[c][1] = 0.0;
+
+  double rpay[PER], rx = 0.0, ry = 0.0;
+  auto fetch = [&](int64_t base) {
+    // sources past the end: far away and weightless
+    if (tid < kWfSrc) {
+      const int64_t j = base + tid;
+      rx = j < p.n ? p.src[2 * j] : 1e100;
+      ry = j < p.n ? p.src[2 * j + 1] : 1e100;
+    }
+#pragma unroll
+    for (int q = 0; q < PER; q++) {
+      const int e = tid + 256 * q;               // (source, set, component), component fastest: coalesced
+      const int64_t j = base + e / (2 * NC);
+      rpay[q] = j < p.n ? p.area[j] * p.J[j * p.ldv + 2 * p.rhs0 + e % (2 * NC)] : 0.0;
+    }
+  };
+  auto stash = [&](int buf) {
+    if (tid < kWfSrc) {
+      sx[buf][tid] = rx;
+      sy[buf][tid] = ry;
+    }
+#pragma unroll
+    for (int q = 0; q < PER; q++) {
+      const int e = tid + 256 * q;
+      const int jl = e / (2 * NC), sc = e % (2 * NC);
+      sp[buf][(2 * jl + (sc & 1)) * PLD + (sc >> 1)] = rpay[q];
+    }
+  };
+  fetch(0);
+  stash(0);
+  __syncthreads();
+  int buf = 0;
+  for (int64_t base = 0; base < p.n; base += kWfSrc) {
+    const bool more = base + kWfSrc < p.n;
+    if (more) fetch(base + kWfSrc);
+#pragma unroll
+    for (int kk = 0; kk < kWfSrc / 4; kk++) {
+      const int j = kk * 4 + t;
+      const double dx = tx - sx[buf][j], dy = ty - sy[buf][j];
+      const double k3 = inv_r3(fma(dx, dx, dy * dy));
+      const double ay = k3 * dy, ax = -(k3 * dx);
+#pragma unroll
+      for (int h = 0; h < 2; h++) {
+        const int from = (lane & ~3) | (2 * h + (t >> 1));
+        const double vy = __shfl_sync(0xffffffffu, ay, from);
+        const double vx = __shfl_sync(0xffffffffu, ax, from);
+        const double a = (t & 1) ? vx : vy;
+        const int krow = (kk * 2 + h) * 4 + t;
+#pragma unroll
+        for (int c = 0; c < CT; c++) dmma_nb(acc[c][0], acc[c][1], a, sp[buf][krow * PLD + c * 8 + g]);
+      }
+    }
+    if (more) stash(buf ^ 1);
+    __syncthreads();
+    buf ^= 1;
+  }
+  if (!active) return;
+  const double pf = p.prefactor;
+#pragma unroll
+  for (int c = 0; c < CT; c++)
+#pragma unroll
+    for (int e = 0; e < 2; e++) p.out[i * p.ldo + p.rhs0 + c * 8 + 2 * t + e] = pf * acc[c][e];
+}
+
+// Sets per pass of within_film_gemm_kernel in scb_biot_savart_within_film.  Measured on a B200 (1000 W limit)
+// at 20k vertices x 40k triangles against 8-set CUDA-core passes: 0.71x at 16 sets, 1.01x at 32, 1.17x at 64
+// (DESIGN.md 4.5), so only full 64-set passes use it.
+constexpr int64_t kWithinFilmGemmSets = 64;
+
 // out[i, rhs0..] (+)= prefactor * sum_{j in src, r_ij > 0} q_ij w_j v[j, rhs0..]
 int nbody_kernel_sum(int64_t m, const double* tgt, int64_t n, const double* src,
                      const int64_t* src_idx, const double* w, const double* v, int64_t ldv,
@@ -501,6 +609,22 @@ extern "C" int scb_biot_savart(int kind, int64_t m, const double* tgt, int64_t n
     SCB_CUDA(cudaMemsetAsync(out, 0, sizeof(double) * (size_t)(m * ocomp * nsets), s));
     return SCB_OK;
   }
+  if (kind == SCB_BS_BOUNDARY) {
+    // edge geometry shared by every set: strengths area[n, nsets], out[m, nsets]
+    NbodyParams p{};
+    p.m = m; p.tgt = tgt; p.n = n; p.src = src; p.area = area; p.J = J;
+    p.ldv = nsets; p.ldo = nsets; p.prefactor = prefactor; p.out = out;
+    for (int64_t k = 0; k < nsets;) {
+      p.rhs0 = k;
+      int rc;
+      if (nsets - k >= 8) { rc = launch_nbody<NB_BOUNDARY, 8>(p, s); k += 8; }
+      else if (nsets - k >= 4) { rc = launch_nbody<NB_BOUNDARY, 4>(p, s); k += 4; }
+      else if (nsets - k >= 2) { rc = launch_nbody<NB_BOUNDARY, 2>(p, s); k += 2; }
+      else { rc = launch_nbody<NB_BOUNDARY, 1>(p, s); k += 1; }
+      if (rc) return rc;
+    }
+    return SCB_OK;
+  }
   int64_t k = 0;
   while (k < nsets) {
     NbodyParams p{};
@@ -519,7 +643,6 @@ extern "C" int scb_biot_savart(int kind, int64_t m, const double* tgt, int64_t n
       case SCB_BS_Z: rc = launch_nbody<NB_Z, 1>(p, s); break;
       case SCB_BS_VECTOR: rc = launch_nbody<NB_VECTOR, 1>(p, s); break;
       case SCB_BS_VECTOR_POTENTIAL: rc = launch_nbody<NB_VECPOT, 1>(p, s); break;
-      case SCB_BS_BOUNDARY: rc = launch_nbody<NB_BOUNDARY, 1>(p, s); break;
       default: set_error("scb_biot_savart: unknown kind %d", kind); return SCB_ERR_INVALID;
     }
     if (rc) return rc;
@@ -542,7 +665,39 @@ extern "C" int scb_film_coupling(int64_t m, const double* tgt, double tgt_z, int
   NbodyParams p{};
   p.m = m; p.tgt = tgt; p.tgt_z = tgt_z; p.n = n; p.src = src; p.area = area; p.J = J; p.ldv = 2 * nsets;
   p.skip_lo = skip_lo; p.skip_len = skip_hi - skip_lo; p.prefactor = prefactor; p.out = out; p.ldo = nsets;
+  p.sld = 3;
   int64_t k = 0;
+  while (k < nsets) {
+    p.rhs0 = k;
+    int rc;
+    if (nsets - k >= 8) { rc = launch_nbody<NB_COUPLING, 8>(p, s); k += 8; }
+    else if (nsets - k >= 4) { rc = launch_nbody<NB_COUPLING, 4>(p, s); k += 4; }
+    else if (nsets - k >= 2) { rc = launch_nbody<NB_COUPLING, 2>(p, s); k += 2; }
+    else { rc = launch_nbody<NB_COUPLING, 1>(p, s); k += 1; }
+    if (rc) return rc;
+  }
+  return SCB_OK;
+}
+
+extern "C" int scb_biot_savart_within_film(int64_t m, const double* tgt, int64_t n, const double* src,
+                                           const double* area, const double* J, double prefactor, int64_t nsets,
+                                           double* out, scb_stream_t stream) {
+  SCB_CHECK_ARG(m >= 0 && n >= 0 && nsets >= 1, "bad sizes");
+  cudaStream_t s = (cudaStream_t)stream;
+  if (m == 0) return SCB_OK;
+  if (n == 0) {
+    SCB_CUDA(cudaMemsetAsync(out, 0, sizeof(double) * (size_t)(m * nsets), s));
+    return SCB_OK;
+  }
+  NbodyParams p{};
+  p.m = m; p.tgt = tgt; p.n = n; p.src = src; p.area = area; p.J = J; p.ldv = 2 * nsets; p.ldo = nsets;
+  p.sld = 2; p.prefactor = prefactor; p.out = out;  // (NB_COUPLING: sources in the target plane, nothing skipped)
+  int64_t k = 0;
+  for (; nsets - k >= kWithinFilmGemmSets; k += kWithinFilmGemmSets) {
+    p.rhs0 = k;
+    within_film_gemm_kernel<kWithinFilmGemmSets / 8><<<(unsigned)ceil_div(m, 64), 256, 0, s>>>(p);
+    SCB_LAUNCH_CHECK();
+  }
   while (k < nsets) {
     p.rhs0 = k;
     int rc;

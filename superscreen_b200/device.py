@@ -664,7 +664,9 @@ class Device:
         for compatibility (there is no per-hole loop to show progress of).  The reference solves once
         per driven hole against one factorization; here all columns are one batched solve
         (``solve_batch``).  As in the reference, ``iterations`` is forwarded to the solver only if
-        given explicitly (SURVEY.md Q8)."""
+        given explicitly (SURVEY.md Q8).  Films with transport terminals are solved as the reference solves
+        them, with zero terminal currents: their boundary stays out of the linear system and their self
+        field is the Biot-Savart sum over their triangles."""
         from .solver import factorize_model, solve_batch
 
         from . import _lib

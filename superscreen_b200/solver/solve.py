@@ -22,7 +22,8 @@ from ..device import Device
 from ..solution import FilmSolution, Solution, Vortex
 from ..sources import ConstantField
 from .solve_film import (  # noqa: F401  (TerminalSystems, solve_film: names the reference module exposes)
-    LinearSystem, TerminalSystems, factorize_linear_systems, hole_boundary_state, solve_film, solve_film_device)
+    LinearSystem, TerminalSystems, factorize_linear_systems, hole_boundary_state, solve_film, solve_film_device,
+    terminal_transport_state)
 from .utils import FilmInfo, currents_to_floats, field_conversion_factor, make_film_info
 
 logger = logging.getLogger("solve")
@@ -264,9 +265,11 @@ def _packed_sources(model: "FactorizedModel", layout, z0s, dev):
 
 
 def _run(model: "FactorizedModel", applied_fields, circ_by_film, vortex_flux, iterations, check_inversion,
-         field_conversion: float, batch: Optional[int] = None, last_only: bool = False, gather: bool = True):
+         field_conversion: float, batch: Optional[int] = None, last_only: bool = False, gather: bool = True,
+         terminal_currents: Optional[List[Dict[str, Dict[str, float]]]] = None):
     """Runs the solve + film-to-film iterations on the device for single or batched right-hand
-    sides.  Everything stays on the device until the end: every owned film's result of every stored
+    sides.  ``terminal_currents`` (batched only): one ``{film: {terminal: current}}`` dict per entry
+    (default: the model's for every entry).  Everything stays on the device until the end: every owned film's result of every stored
     iterate is packed into one buffer (``parallel.ResultPacker``), replicated over the ranks by one
     all-gather if ``gather`` and downloaded once.  Returns ``parallel.HostResults``."""
     torch = _torch()
@@ -289,6 +292,7 @@ def _run(model: "FactorizedModel", applied_fields, circ_by_film, vortex_flux, it
     iterates = [n_solutions - 1] if last_only else list(range(n_solutions))
 
     hole_states = {}  # hole boundary values + their effective field: constant over the iterations
+    transport_states = {}  # terminal films: transport stream + its boundary field, constant likewise
     n_solves = {}     # per film: number of the iterate being solved (the driver solves every film once per iterate)
 
     def solve_fn(name, other):
@@ -304,12 +308,22 @@ def _run(model: "FactorizedModel", applied_fields, circ_by_film, vortex_flux, it
             hole_states[name] = hole_boundary_state(
                 info, model.hole_systems[name], info.circulating_currents if circ is None else circ,
                 applied_fields[name]) if model.hole_systems[name] else (None, None)
+        terminal_systems = model.terminal_systems.get(name)
+        if terminal_systems is not None and name not in transport_states:
+            info = film_info[name]
+            if terminal_currents is not None:
+                currents = [tc.get(name, {}) for tc in terminal_currents]
+            else:
+                currents = info.terminal_currents or {}
+                if batch is not None:
+                    currents = [currents] * batch
+            transport_states[name] = terminal_transport_state(device, info, terminal_systems, currents)
         return solve_film_device(
             film_info=film_info[name], film_system=model.film_systems[name],
             hole_systems=model.hole_systems[name], applied_field=applied_fields[name], vortex_flux=vortex_flux,
             field_from_other_films=other, check_inversion=check_inversion, circulating_currents=circ,
-            terminal_systems=model.terminal_systems.get(name), device=device, hole_state=hole_states[name],
-            want_self_field=it in iterates)  # (the self field of an iterate that is not stored is never used)
+            terminal_systems=terminal_systems, device=device, hole_state=hole_states[name],
+            transport_state=transport_states.get(name), want_self_field=it in iterates)  # (the self field of an iterate that is not stored is never used)
 
     inv4pi = 1.0 / (4.0 * np.pi)
 
@@ -429,8 +443,41 @@ def solve(device: Optional[Device] = None, *, model: Optional[FactorizedModel] =
     return solutions
 
 
+def _batch_terminal_currents(model: FactorizedModel, terminal_currents, B: int):
+    """Validates and converts the per-entry terminal currents of ``solve_batch`` exactly as
+    ``factorize_model`` + ``solve`` would (before any device work): floats or unit strings in
+    ``model.current_units``, known films and terminals, conserved per film, and -- as the stream
+    function needs it -- every terminal of a film that carries a current."""
+    device = model.device
+    if len(terminal_currents) != B:
+        raise ValueError("applied_fields and terminal_currents must have the same length.")
+    out = []
+    for entry in terminal_currents:
+        entry = entry or {}
+        converted = {}
+        for film_name, currents in entry.items():
+            if film_name not in device.terminals:
+                raise KeyError(f"terminal_currents contains a film without terminals: {film_name!r}")
+            names = [t.name for t in device.terminals[film_name]]
+            diff = set(currents) - set(names)
+            if diff:
+                raise KeyError(f"terminal_currents[{film_name!r}] contains unknown terminals: {sorted(diff)!r}")
+            currents = currents_to_floats(currents, device.ureg, model.current_units)
+            if sum(currents.values()):
+                raise ValueError(f"Terminal currents in film {film_name!r} are not conserved.")
+            if any(currents.values()):
+                missing = [name for name in names if name not in currents]
+                if missing:
+                    raise KeyError(missing[0])
+            converted[film_name] = currents
+        out.append(converted)
+    return out
+
+
 def solve_batch(*, model: FactorizedModel, applied_fields: Sequence[Optional[Callable]],
-                circulating_currents: Optional[Sequence[Dict[str, float]]] = None, field_units: str = "mT",
+                circulating_currents: Optional[Sequence[Dict[str, float]]] = None,
+                terminal_currents: Optional[Sequence[Dict[str, Dict[str, Union[float, str]]]]] = None,
+                field_units: str = "mT",
                 iterations: int = 0, check_inversion: bool = False, last_only: bool = False,
                 gather: bool = True, _solver: str = "superscreen_b200.solve_batch") -> List[List[Solution]]:
     """Solves B models that share one factorization in a single batched pass (multi-RHS getrs,
@@ -440,7 +487,12 @@ def solve_batch(*, model: FactorizedModel, applied_fields: Sequence[Optional[Cal
     (e.g. once per driven hole in ``Device.mutual_inductance_matrix``, device/device.py:610-639, or
     once per applied field in a sweep).  ``out[b]`` equals
     ``solve(model=model_b, applied_field=applied_fields[b], iterations=iterations)`` where
-    ``model_b`` has ``circulating_currents[b]`` (floats in ``model.current_units``).  With
+    ``model_b`` is ``model`` factorized with ``circulating_currents[b]`` (floats in ``model.current_units``)
+    and ``terminal_currents[b]``.  ``terminal_currents`` has one ``{film: {terminal: current}}`` dict per
+    entry (floats in ``model.current_units`` or unit strings; default: ``model.terminal_currents`` for
+    every entry); an entry replaces the model's terminal currents completely: films it does not name
+    carry no transport current.  The transport stream of every entry is computed once per call, with
+    one column per entry in every device operation.  With
     ``last_only`` only the final iterate is brought to the host (``out[b]`` has one element).
     With a multi-rank model, ``gather=False`` skips the replication of the results: every rank's
     solutions then hold only the films it owns (enough for per-film post-processing such as the
@@ -460,6 +512,8 @@ def solve_batch(*, model: FactorizedModel, applied_fields: Sequence[Optional[Cal
         diff = set(cc) - set(device.holes)
         if diff:
             raise KeyError(f"circulating_currents contains keys not in self.device.holes: {list(diff)!r}")
+    if terminal_currents is not None:
+        terminal_currents = _batch_terminal_currents(model, terminal_currents, B)
     current_units = model.current_units
     length_units = device.length_units
     field_conversion = field_conversion_factor(field_units, current_units, length_units=length_units).magnitude
@@ -503,10 +557,11 @@ def solve_batch(*, model: FactorizedModel, applied_fields: Sequence[Optional[Cal
                                   if film == name}
     vortex_flux = _u.PHI_0 / _u.MU_0 * _u.conversion_factor("A * m", f"({current_units}) * ({length_units})")
     host = _run(model, dev_fields, circ_by_film, vortex_flux, iterations, check_inversion, field_conversion,
-                batch=B, last_only=last_only, gather=gather)
+                batch=B, last_only=last_only, gather=gather, terminal_currents=terminal_currents)
     kwargs_list = [dict(applied_field_func=funcs[b], field_units=field_units, current_units=current_units,
                         circulating_currents=dict(circulating_currents[b]),
-                        terminal_currents=model.terminal_currents, vortices=model.vortices, solver=_solver)
+                        terminal_currents=model.terminal_currents if terminal_currents is None
+                        else terminal_currents[b], vortices=model.vortices, solver=_solver)
                    for b in range(B)]
     with _lib.nvtx_range("scb.solve_batch.solutions"):
         per_iter_solutions = _solutions_from_host(device, host, film_names, host_fields, field_conversion,

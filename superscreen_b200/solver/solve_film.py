@@ -423,7 +423,8 @@ def hole_boundary_state(film_info: FilmInfo, hole_systems: Dict[str, LinearSyste
 def solve_film_device(*, film_info: FilmInfo, film_system: LinearSystem, hole_systems: Dict[str, LinearSystem],
                       applied_field, vortex_flux: float, field_from_other_films=None,
                       check_inversion: bool = False, circulating_currents=None, terminal_systems=None,
-                      device: Optional[Device] = None, hole_state=None, want_self_field: bool = True):
+                      device: Optional[Device] = None, hole_state=None, want_self_field: bool = True,
+                      terminal_currents=None, transport_state=None):
     """Device-side body of ``solve_film`` (reference solve_film.py:483-565): all arguments and
     results are device tensors in solver units.  ``want_self_field=False`` skips the screening mat-vec
     ``Q @ (w g)`` (an output only: the next Jacobi step needs ``J``, not the self field) and returns
@@ -432,7 +433,9 @@ def solve_film_device(*, film_info: FilmInfo, film_system: LinearSystem, hole_sy
     ``applied_field`` is ``(n,)`` or, for a batch of B right-hand sides sharing the factorization,
     ``(n, B)``; ``circulating_currents`` (default: ``film_info.circulating_currents``) maps hole
     names to a float or to a ``(B,)`` tensor.  ``hole_state`` = ``hole_boundary_state(...)`` if the
-    caller has it already.  Returns ``(g, J, self_field)`` with shapes ``(n,), (n, 2), (n,)`` or
+    caller has it already.  For a film with transport terminals, ``terminal_currents`` (default:
+    ``film_info.terminal_currents``) is one ``{terminal: current}`` dict, or a sequence of B of them for a
+    batch, and ``transport_state`` = ``terminal_transport_state(...)`` if the caller has it already.  Returns ``(g, J, self_field)`` with shapes ``(n,), (n, 2), (n,)`` or
     ``(n, B), (n, B, 2), (n, B)``.
     """
     torch = _torch()
@@ -486,26 +489,16 @@ def solve_film_device(*, film_info: FilmInfo, film_system: LinearSystem, hole_sy
             g = torch.zeros_like(Hz) if g0 is None else g0.clone()
             if transport:
                 # reference solve_film.py:505-524
-                if batched:
-                    raise NotImplementedError("Batched right-hand sides are not supported for terminal films.")
-                g_transport = solve_for_terminal_current_stream(device, info, terminal_systems,
-                                                                info.terminal_currents or {})
-                g = g + g_transport
-                b = terminal_systems.boundary.indices_dev
-                boundary_sites = d.sites[b]
-                boundary_stream = g_transport[b]
-                centers = (0.5 * (boundary_sites + torch.roll(boundary_sites, -1, dims=0))).contiguous()
-                boundary_stream = 0.5 * (boundary_stream + torch.roll(boundary_stream, -1, dims=0))
-                dr = torch.roll(boundary_sites, -1, dims=0) - boundary_sites  # edges of the closed curve
-                lengths = torch.linalg.norm(dr, dim=1)
-                normals = (torch.stack([dr[:, 1], -dr[:, 0]], dim=1) / lengths[:, None]).contiguous()
-                Ha_transport = torch.empty(d.n, dtype=torch.float64, device=d.device)
-                # _get_boundary_effective_field (solve_film.py:393-412): kind 4, area = stream * length
-                _lib.check(L.scb_biot_savart(
-                    4, d.n, _lib.ptr(d.sites), int(b.numel()), _lib.ptr(centers),
-                    _lib.ptr((boundary_stream * lengths).contiguous()), _lib.ptr(normals), 0.0, 1.0 / (4.0 * np.pi), 1,
-                    _lib.ptr(Ha_transport), _lib.stream_ptr()))
-                Ha_eff = Ha_transport if Ha_eff is None else Ha_eff + Ha_transport
+                if transport_state is None:
+                    if terminal_currents is None:
+                        terminal_currents = info.terminal_currents or {}
+                    if batched and isinstance(terminal_currents, dict):
+                        terminal_currents = [terminal_currents] * nrhs
+                    transport_state = terminal_transport_state(device, info, terminal_systems, terminal_currents)
+                g_transport, Ha_transport = transport_state
+                if g_transport is not None:  # (None: no entry carries a terminal current)
+                    g = g + g_transport
+                    Ha_eff = Ha_transport if Ha_eff is None else Ha_eff + Ha_transport
             ix = film_system.indices_dev
             h = Hz[ix] if Ha_eff is None else Hz[ix] - Ha_eff[ix]
             gf = lu_solve(film_system, h)
@@ -561,71 +554,143 @@ def solve_film_device(*, film_info: FilmInfo, film_system: LinearSystem, hole_sy
         if not want_self_field:
             self_field = None
         elif transport:
-            # _biot_savart_within_film on per-triangle current densities (solve_film.py:557-562)
-            J_tri = torch.stack([spmv(d, "gtri_y", g), spmv(d, "gtri_x", g, alpha=-1.0)], dim=1).contiguous()
-            self_field = torch.empty(d.n, dtype=torch.float64, device=d.device)
-            _lib.check(L.scb_biot_savart(
-                0, d.n, _lib.ptr(d.sites), d.m, _lib.ptr(d.t["centroids"]), _lib.ptr(d.t["triangle_areas"]),
-                _lib.ptr(J_tri), 0.0, 1.0 / (4.0 * np.pi), 1, _lib.ptr(self_field), _lib.stream_ptr()))
+            # _biot_savart_within_film on per-triangle current densities (solve_film.py:557-562):
+            # J_tri [m, nsets, 2] source-major
+            J_tri = torch.stack([spmv(d, "gtri_y", g), spmv(d, "gtri_x", g, alpha=-1.0)], dim=-1).contiguous()
+            self_field = torch.empty(g.shape, dtype=torch.float64, device=d.device)
+            _lib.check(L.scb_biot_savart_within_film(
+                d.n, _lib.ptr(d.sites), d.m, _lib.ptr(d.t["centroids"]), _lib.ptr(d.t["triangle_areas"]),
+                _lib.ptr(J_tri), 1.0 / (4.0 * np.pi), nrhs, _lib.ptr(self_field), _lib.stream_ptr()))
         else:
             # Q @ (w * g), matrix-free
             self_field = apply_operator(info, g, src_idx=None, with_sparse=False)
     return g, J, self_field
 
 
-def solve_for_terminal_current_stream(device: Device, film_info: FilmInfo, terminal_systems: TerminalSystems,
-                                      terminal_currents: Dict[str, float]):
-    """reference solver/solve_film.py:308-390.  The boundary values are a few hundred numbers and
-    are set on the host exactly as the reference does; the slab products ``A_boundary @ g`` and
-    ``A_hole @ g`` are matrix-free device operations and the two solves use the device LUs."""
-    torch = _torch()
+def _terminal_boundary_values(device: Device, film_info: FilmInfo, terminal_systems: TerminalSystems,
+                              columns) -> Optional[np.ndarray]:
+    """Host part of reference solver/solve_film.py:308-335 for every ``{terminal: current}`` dict in
+    ``columns``: the stream function on the (counter-clockwise) boundary, shifted by
+    ``- max(g) + ptp(g) / 2`` per column.  Returns ``(n_boundary + 1, B)``: the boundary values and, in
+    the last row, the value the shift gives every other vertex; a column without current is all zero.
+    ``None`` when no column carries a current."""
     from .utils import stream_from_terminal_current
 
-    d = film_info.mesh._data
+    if not any(any(c.values()) for c in columns):
+        return None
     points = film_info.mesh.sites
-    npoints = len(points)
-    if not any(terminal_currents.values()):
-        return torch.zeros(npoints, dtype=torch.float64, device=d.device)
-    terminals = list(device.terminals[film_info.name])
     boundary_indices = terminal_systems.boundary.indices
-    boundary_points = points[boundary_indices]
-    # 1. stream function on the boundary
-    g = np.zeros(npoints)
-    for terminal in terminals:
-        current = terminal_currents[terminal.name]
-        ix_boundary = np.sort(terminal.contains_points(boundary_points, index=True))
-        remaining_boundary = boundary_indices[ix_boundary[-1]:]
-        ix_terminal = boundary_indices[ix_boundary]
-        stream = stream_from_terminal_current(points[ix_terminal], -current)
-        g[ix_terminal[:-1]] += stream
-        g[remaining_boundary] += stream[-1]
-    g = g - np.max(g) + np.ptp(g) / 2
+    nb = len(boundary_indices)
+    out = np.zeros((nb + 1, len(columns)))
+    # per terminal: its boundary positions (ascending) -- the same for every column
+    ix_by_terminal = {t.name: np.sort(t.contains_points(points[boundary_indices], index=True))
+                      for t in device.terminals[film_info.name]}
+    for k, terminal_currents in enumerate(columns):
+        if not any(terminal_currents.values()):
+            continue
+        g = np.zeros(nb + 1)  # (boundary positions; the last entry stands for every other vertex)
+        for name, ix_boundary in ix_by_terminal.items():
+            current = terminal_currents[name]
+            stream = stream_from_terminal_current(points[boundary_indices[ix_boundary]], -current)
+            g[ix_boundary[:-1]] += stream
+            g[ix_boundary[-1]:nb] += stream[-1]
+        out[:, k] = g - np.max(g) + np.ptp(g) / 2
+    return out
+
+
+def solve_for_terminal_current_stream(device: Device, film_info: FilmInfo, terminal_systems: TerminalSystems,
+                                      terminal_currents):
+    """reference solver/solve_film.py:308-390 for one ``{terminal: current}`` dict -> ``(n,)``, or for a
+    sequence of B of them -> ``(n, B)``.  The boundary values are a few hundred numbers per column and
+    are set on the host exactly as the reference does (one upload for the whole batch); the slab products
+    ``A_boundary @ g`` and ``A_hole @ g``, the hole averages and the two solves run on the device with
+    one column per entry.  Returns the device tensor."""
+    torch = _torch()
+    batched = not isinstance(terminal_currents, dict)
+    columns = list(terminal_currents) if batched else [terminal_currents]
+    d = film_info.mesh._data
+    values = _terminal_boundary_values(device, film_info, terminal_systems, columns)
     with torch.cuda.device(d.device):
+        if values is None:
+            g_dev = torch.zeros(d.n, len(columns), dtype=torch.float64, device=d.device)
+            return g_dev if batched else g_dev[:, 0]
+        values = torch.as_tensor(values).to(d.device)
         b_dev = terminal_systems.boundary.indices_dev
-        g_dev = torch.as_tensor(g).to(d.device)
+        nb = int(b_dev.numel())
+        g_dev = values[nb:].expand(d.n, -1).clone()
+        g_dev[b_dev] = values[:nb]
         # only the boundary entries enter A_boundary @ g[boundary] (the constant shift above also
         # moved the interior entries, which the solve below overwrites)
         v = torch.zeros_like(g_dev)
-        v[b_dev] = g_dev[b_dev]
+        v[b_dev] = values[:nb]
         Ha_eff = -apply_operator(film_info, v, src_idx=b_dev)
         # 2. interior ignoring the holes
         sys_all = terminal_systems.film_without_boundary
         g_dev[sys_all.indices_dev] = lu_solve(sys_all, -Ha_eff[sys_all.indices_dev])
-        if len(terminal_systems.holes) == 0:
-            return g_dev
-        # 3. holes at the weighted average of step 2, then the interior without holes
-        w = d.t["vertex_areas"]
-        v = torch.zeros_like(g_dev)
-        v[b_dev] = g_dev[b_dev]
-        for system in terminal_systems.holes.values():
-            ixh = system.indices_dev
-            g_dev[ixh] = (g_dev[ixh] * w[ixh]).sum() / w[ixh].sum()
-            v[ixh] = g_dev[ixh]
-        src = torch.cat([b_dev] + [s.indices_dev for s in terminal_systems.holes.values()])
-        Ha_eff = -apply_operator(film_info, v, src_idx=src)
-        sys_nh = terminal_systems.film_without_boundary_or_holes
-        g_dev[sys_nh.indices_dev] = lu_solve(sys_nh, -Ha_eff[sys_nh.indices_dev])
-    return g_dev
+        if len(terminal_systems.holes):
+            # 3. holes at the weighted average of step 2, then the interior without holes
+            w = d.t["vertex_areas"]
+            for system in terminal_systems.holes.values():
+                ixh = system.indices_dev
+                v[ixh] = ((g_dev[ixh] * w[ixh, None]).sum(dim=0) / w[ixh].sum())[None, :]
+                g_dev[ixh] = v[ixh]
+            src = torch.cat([b_dev] + [s.indices_dev for s in terminal_systems.holes.values()])
+            Ha_eff = -apply_operator(film_info, v, src_idx=src)
+            sys_nh = terminal_systems.film_without_boundary_or_holes
+            g_dev[sys_nh.indices_dev] = lu_solve(sys_nh, -Ha_eff[sys_nh.indices_dev])
+    return g_dev if batched else g_dev[:, 0]
+
+
+def _boundary_geometry(film_info: FilmInfo, terminal_systems: TerminalSystems):
+    """Edge centres, lengths and unit normals of the closed boundary curve (reference
+    solve_film.py:510-518); cached with the film's other index-set derived arrays."""
+    torch = _torch()
+    d = film_info.mesh._data
+    geo = film_info.dev.get("_geo")
+    key = ("boundary_edges", str(d.device))
+    hit = None if geo is None else geo.get(key)
+    if hit is None:
+        b = terminal_systems.boundary.indices_dev
+        boundary_sites = d.sites[b]
+        centers = (0.5 * (boundary_sites + torch.roll(boundary_sites, -1, dims=0))).contiguous()
+        dr = torch.roll(boundary_sites, -1, dims=0) - boundary_sites  # edges of the closed curve
+        lengths = torch.linalg.norm(dr, dim=1)
+        normals = (torch.stack([dr[:, 1], -dr[:, 0]], dim=1) / lengths[:, None]).contiguous()
+        hit = (centers, lengths, normals)
+        if geo is not None:
+            geo[key] = hit
+    return hit
+
+
+def terminal_transport_state(device: Device, film_info: FilmInfo, terminal_systems: TerminalSystems,
+                             terminal_currents):
+    """Transport part of a terminal film's solve (reference solve_film.py:505-524): the stream function
+    of the terminal currents and the effective field of its boundary values.  Depends neither on the
+    applied field nor on the film-to-film iterate: evaluated once per solve call.  ``terminal_currents``
+    is one ``{terminal: current}`` dict (results ``(n,)``) or a sequence of B of them (``(n, B)``).
+    Returns ``(g_transport, Ha_transport)``, or ``(None, None)`` when no entry carries a current."""
+    torch = _torch()
+    L = _lib.lib()
+    batched = not isinstance(terminal_currents, dict)
+    columns = list(terminal_currents) if batched else [terminal_currents]
+    if not any(any(c.values()) for c in columns):
+        return None, None
+    d = film_info.mesh._data
+    with torch.cuda.device(d.device):
+        g_transport = solve_for_terminal_current_stream(device, film_info, terminal_systems, columns)
+        b = terminal_systems.boundary.indices_dev
+        centers, lengths, normals = _boundary_geometry(film_info, terminal_systems)
+        boundary_stream = g_transport[b]
+        boundary_stream = 0.5 * (boundary_stream + torch.roll(boundary_stream, -1, dims=0))
+        Ha_transport = torch.empty(d.n, len(columns), dtype=torch.float64, device=d.device)
+        # _get_boundary_effective_field (solve_film.py:393-412): kind 4, strengths = stream * length [nb, B]
+        _lib.check(L.scb_biot_savart(
+            4, d.n, _lib.ptr(d.sites), int(b.numel()), _lib.ptr(centers),
+            _lib.ptr((boundary_stream * lengths[:, None]).contiguous()), _lib.ptr(normals), 0.0,
+            1.0 / (4.0 * np.pi), len(columns), _lib.ptr(Ha_transport), _lib.stream_ptr()))
+    if not batched:
+        return g_transport[:, 0], Ha_transport[:, 0]
+    return g_transport, Ha_transport
 
 
 def solve_film(*, device: Device, applied_field: np.ndarray, film_info: FilmInfo, film_system: LinearSystem,
