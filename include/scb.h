@@ -280,6 +280,36 @@ int scb_solve_step(int64_t n, int64_t n_int, int64_t n_pad, int64_t nrhs, const 
                    const double* gradient_y, double* J, scb_stream_t stream);
 
 /* ------------------------------------------------------------------------------------
+ * Vortices (solver/solve_film.py:541-554).  The vortex term of the reference,
+ *   g[ix] += flux nPhi0 K[:, j_film] / w[j_device],   K = -(-A)^-1,
+ * is the solution of (-A) x = h - c e_{j_film} with c = flux nPhi0 / w[j_device]: a sparse correction to
+ * the right-hand side, applied between scb_solve_rhs and scb_getrs_nopiv (or to h itself before a
+ * solve), with no solve of its own.  A film with vortices runs
+ *   scb_solve_rhs -> scb_vortex_rhs -> scb_getrs_nopiv -> scb_solve_stream -> scb_current_density.
+ * ------------------------------------------------------------------------------------ */
+
+/* Nearest vertex of each of the nv query points xy [nv, 2] among the n_sub sites sites[sub[k]]
+ * (j_sub [nv] <- k: the system row j_film for sub = the system's index set) and among all n sites
+ * (j_all [nv] <- i: j_device), in one pass.  Bit for bit np.argmin(np.linalg.norm(P - xy, axis=1)): the
+ * distances are rounded as numpy rounds them (sqrt(dx*dx + dy*dy), no FMA contraction), the ROUNDED
+ * distances are compared (distinct squared distances can round to one norm), ties and NaN resolve as in
+ * numpy (lowest index).  The reduction runs on (distance, index) pairs under that total order: the result
+ * does not depend on its order.  sub, j_sub, j_all are int64.  nv = 0 does nothing; otherwise n, n_sub >= 1. */
+int scb_locate_vortices(int64_t nv, const double* xy, int64_t n, const double* sites, int64_t n_sub,
+                        const int64_t* sub, int64_t* j_sub, int64_t* j_all, scb_stream_t stream);
+
+/* Vortex right-hand-side terms of nrhs columns.  The vortices are sorted by column in a CSR layout:
+ * column c holds vortices col_ptr[c] .. col_ptr[c+1] (int64 [nrhs+1]).  For each of them, in order,
+ *   B[row[v], c] -= flux * nphi0[v] / weights[j_all[v]] * scale[row[v]]
+ * (one rounding per operation, left to right; B [rows, nrhs] row-major).  `row` is the row of B, not the
+ * vertex: j_sub of scb_locate_vortices, or for a pivoted system (B[r] = h[perm[r]]) invperm[j_sub].
+ * scale (NULL: not symmetrised) is the D of the symmetrised system.  One thread per column, no atomics:
+ * deterministic, and two vortices at one vertex simply add.  row, j_all are int64 [nv]. */
+int scb_vortex_rhs(int64_t nrhs, const int64_t* col_ptr, const int64_t* row, const int64_t* j_all,
+                   const double* nphi0, const double* weights, double flux, const double* scale, double* B,
+                   scb_stream_t stream);
+
+/* ------------------------------------------------------------------------------------
  * Biot-Savart family (K15-K18, rows a14, a15, a17, a18)
  * ------------------------------------------------------------------------------------ */
 enum scb_bs_kind {

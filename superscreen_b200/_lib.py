@@ -61,6 +61,8 @@ EXPORTS = {
     "scb_solve_stream": (c_int, [c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "scb_current_density": (c_int, [c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
     "scb_solve_step": (c_int, [c_int64, c_int64, c_int64, c_int64] + [c_void_p] * 17),
+    "scb_locate_vortices": (c_int, [c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "scb_vortex_rhs": (c_int, [c_int64] + [c_void_p] * 5 + [c_double, c_void_p, c_void_p, c_void_p]),
     "scb_biot_savart": (c_int, [c_int, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_double, c_double, c_int64, c_void_p, c_void_p]),
     "scb_film_coupling": (c_int, [c_int64, c_void_p, c_double, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_int64,
                                   c_double, c_int64, c_void_p, c_void_p]),

@@ -22,9 +22,10 @@ from ..device import Device
 from ..solution import FilmSolution, Solution, Vortex
 from ..sources import ConstantField
 from .solve_film import (  # noqa: F401  (TerminalSystems, solve_film: names the reference module exposes)
-    LinearSystem, TerminalSystems, factorize_linear_systems, hole_boundary_state, solve_film, solve_film_device,
-    terminal_transport_state)
-from .utils import FilmInfo, currents_to_floats, field_conversion_factor, make_film_info
+    LinearSystem, TerminalSystems, factorize_linear_systems, hole_boundary_state, make_vortex_state, solve_film,
+    solve_film_device, terminal_transport_state)
+from .utils import (FilmInfo, currents_to_floats, field_conversion_factor, get_holes_and_vortices_by_film,
+                    make_film_info)
 
 logger = logging.getLogger("solve")
 
@@ -266,11 +267,13 @@ def _packed_sources(model: "FactorizedModel", layout, z0s, dev):
 
 def _run(model: "FactorizedModel", applied_fields, circ_by_film, vortex_flux, iterations, check_inversion,
          field_conversion: float, batch: Optional[int] = None, last_only: bool = False, gather: bool = True,
-         terminal_currents: Optional[List[Dict[str, Dict[str, float]]]] = None):
+         terminal_currents: Optional[List[Dict[str, Dict[str, float]]]] = None,
+         vortices: Optional[List[Dict[str, List[Vortex]]]] = None):
     """Runs the solve + film-to-film iterations on the device for single or batched right-hand
     sides.  ``terminal_currents`` (batched only): one ``{film: {terminal: current}}`` dict per entry
-    (default: the model's for every entry).  Everything stays on the device until the end: every owned film's result of every stored
-    iterate is packed into one buffer (``parallel.ResultPacker``), replicated over the ranks by one
+    (default: the model's for every entry).  ``vortices`` (batched only): one ``{film: [Vortex]}`` dict per
+    entry (default: the model's vortices for every entry).  Everything stays on the device until the
+    end: every owned film's result of every stored iterate is packed into one buffer (``parallel.ResultPacker``), replicated over the ranks by one
     all-gather if ``gather`` and downloaded once.  Returns ``parallel.HostResults``."""
     torch = _torch()
     import contextlib
@@ -293,6 +296,7 @@ def _run(model: "FactorizedModel", applied_fields, circ_by_film, vortex_flux, it
 
     hole_states = {}  # hole boundary values + their effective field: constant over the iterations
     transport_states = {}  # terminal films: transport stream + its boundary field, constant likewise
+    vortex_states = {}     # per film: the located vortices of every column, constant likewise
     n_solves = {}     # per film: number of the iterate being solved (the driver solves every film once per iterate)
 
     def solve_fn(name, other):
@@ -318,12 +322,19 @@ def _run(model: "FactorizedModel", applied_fields, circ_by_film, vortex_flux, it
                 if batch is not None:
                     currents = [currents] * batch
             transport_states[name] = terminal_transport_state(device, info, terminal_systems, currents)
+        if name not in vortex_states:
+            if vortices is not None:
+                columns = [v.get(name, ()) for v in vortices]
+            else:
+                columns = [film_info[name].vortices] * (1 if batch is None else batch)
+            vortex_states[name] = make_vortex_state(film_info[name], model.film_systems[name], columns)
         return solve_film_device(
             film_info=film_info[name], film_system=model.film_systems[name],
             hole_systems=model.hole_systems[name], applied_field=applied_fields[name], vortex_flux=vortex_flux,
             field_from_other_films=other, check_inversion=check_inversion, circulating_currents=circ,
             terminal_systems=terminal_systems, device=device, hole_state=hole_states[name],
-            transport_state=transport_states.get(name), want_self_field=it in iterates)  # (the self field of an iterate that is not stored is never used)
+            transport_state=transport_states.get(name), vortex_state=vortex_states[name],
+            want_self_field=it in iterates)  # (the self field of an iterate that is not stored is never used)
 
     inv4pi = 1.0 / (4.0 * np.pi)
 
@@ -474,9 +485,33 @@ def _batch_terminal_currents(model: FactorizedModel, terminal_currents, B: int):
     return out
 
 
+def _batch_vortices(device: Device, vortices, B: int) -> List[Dict[str, List[Vortex]]]:
+    """Validates the per-entry vortices of ``solve_batch`` with the reference's rules
+    (``get_holes_and_vortices_by_film``: every item a ``Vortex``, in a film of the device, inside that
+    film and not inside one of its holes) before any device work, naming the offending entry.  Returns
+    one ``{film: [Vortex]}`` dict per entry (every film of the device a key)."""
+    if len(vortices) != B:
+        raise ValueError(f"applied_fields and vortices must have the same length (got {B} and {len(vortices)}).")
+    out = []
+    for b, entry in enumerate(vortices):
+        if isinstance(entry, Vortex):
+            raise TypeError(f"vortices[{b}]: expected a sequence of Vortex, but got a single {entry!r}.")
+        entry = [] if entry is None else list(entry)
+        for vortex in entry:
+            if isinstance(vortex, Vortex) and vortex.film not in device.films:
+                raise KeyError(f"vortices[{b}]: {vortex!r} is in a film the device does not have: {vortex.film!r}")
+        try:
+            _, by_film = get_holes_and_vortices_by_film(device, entry)
+        except (TypeError, ValueError) as exc:
+            raise type(exc)(f"vortices[{b}]: {exc}") from exc
+        out.append(by_film)
+    return out
+
+
 def solve_batch(*, model: FactorizedModel, applied_fields: Sequence[Optional[Callable]],
                 circulating_currents: Optional[Sequence[Dict[str, float]]] = None,
                 terminal_currents: Optional[Sequence[Dict[str, Dict[str, Union[float, str]]]]] = None,
+                vortices: Optional[Sequence[Sequence[Vortex]]] = None,
                 field_units: str = "mT",
                 iterations: int = 0, check_inversion: bool = False, last_only: bool = False,
                 gather: bool = True, _solver: str = "superscreen_b200.solve_batch") -> List[List[Solution]]:
@@ -487,12 +522,18 @@ def solve_batch(*, model: FactorizedModel, applied_fields: Sequence[Optional[Cal
     (e.g. once per driven hole in ``Device.mutual_inductance_matrix``, device/device.py:610-639, or
     once per applied field in a sweep).  ``out[b]`` equals
     ``solve(model=model_b, applied_field=applied_fields[b], iterations=iterations)`` where
-    ``model_b`` is ``model`` factorized with ``circulating_currents[b]`` (floats in ``model.current_units``)
-    and ``terminal_currents[b]``.  ``terminal_currents`` has one ``{film: {terminal: current}}`` dict per
-    entry (floats in ``model.current_units`` or unit strings; default: ``model.terminal_currents`` for
+    ``model_b`` is ``model`` factorized with ``circulating_currents[b]`` (floats in ``model.current_units``),
+    ``terminal_currents[b]`` and ``vortices[b]``.  ``terminal_currents`` has one
+    ``{film: {terminal: current}}`` dict per entry (floats in ``model.current_units`` or unit strings; default: ``model.terminal_currents`` for
     every entry); an entry replaces the model's terminal currents completely: films it does not name
     carry no transport current.  The transport stream of every entry is computed once per call, with
-    one column per entry in every device operation.  With
+    one column per entry in every device operation.  ``vortices`` has one sequence of ``Vortex`` per
+    entry (default: ``model.vortices`` for every entry); likewise an entry replaces the model's vortices
+    completely, and an empty sequence (or ``None``) means no vortices.  The vortices are checked as ``factorize_model``
+    checks them (``TypeError`` for an item that is not a ``Vortex``, ``KeyError`` for an unknown film,
+    ``ValueError`` for a vortex outside its film or inside a hole, naming the entry) before any device
+    work.  Each vortex enters its own entry's right-hand side as a sparse correction, so a scan over
+    vortex positions costs one batched solve, not one solve per position.  With
     ``last_only`` only the final iterate is brought to the host (``out[b]`` has one element).
     With a multi-rank model, ``gather=False`` skips the replication of the results: every rank's
     solutions then hold only the films it owns (enough for per-film post-processing such as the
@@ -514,6 +555,10 @@ def solve_batch(*, model: FactorizedModel, applied_fields: Sequence[Optional[Cal
             raise KeyError(f"circulating_currents contains keys not in self.device.holes: {list(diff)!r}")
     if terminal_currents is not None:
         terminal_currents = _batch_terminal_currents(model, terminal_currents, B)
+    vortices_by_film = None
+    if vortices is not None:
+        vortices_by_film = _batch_vortices(device, vortices, B)
+        vortices = [[] if entry is None else list(entry) for entry in vortices]
     current_units = model.current_units
     length_units = device.length_units
     field_conversion = field_conversion_factor(field_units, current_units, length_units=length_units).magnitude
@@ -557,11 +602,13 @@ def solve_batch(*, model: FactorizedModel, applied_fields: Sequence[Optional[Cal
                                   if film == name}
     vortex_flux = _u.PHI_0 / _u.MU_0 * _u.conversion_factor("A * m", f"({current_units}) * ({length_units})")
     host = _run(model, dev_fields, circ_by_film, vortex_flux, iterations, check_inversion, field_conversion,
-                batch=B, last_only=last_only, gather=gather, terminal_currents=terminal_currents)
+                batch=B, last_only=last_only, gather=gather, terminal_currents=terminal_currents,
+                vortices=vortices_by_film)
     kwargs_list = [dict(applied_field_func=funcs[b], field_units=field_units, current_units=current_units,
                         circulating_currents=dict(circulating_currents[b]),
                         terminal_currents=model.terminal_currents if terminal_currents is None
-                        else terminal_currents[b], vortices=model.vortices, solver=_solver)
+                        else terminal_currents[b], vortices=model.vortices if vortices is None else vortices[b],
+                        solver=_solver)
                    for b in range(B)]
     with _lib.nvtx_range("scb.solve_batch.solutions"):
         per_iter_solutions = _solutions_from_host(device, host, film_names, host_fields, field_conversion,

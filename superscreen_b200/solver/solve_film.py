@@ -420,11 +420,79 @@ def hole_boundary_state(film_info: FilmInfo, hole_systems: Dict[str, LinearSyste
     return g0, -apply_operator(film_info, g0, src_idx=src)
 
 
+@dataclass
+class VortexState:
+    """The vortices of one film for every column of a solve, located once per solve call and reused by
+    every film-to-film iteration.  Column ``c`` holds vortices ``col_ptr[c] .. col_ptr[c+1]`` (CSR);
+    ``j_sub`` is each vortex's nearest system row (j_film), ``j_all`` its nearest mesh vertex (j_device)
+    and ``row`` the row of the triangular-solve workspace it enters (``invperm[j_sub]`` for a pivoted
+    system).  All device tensors are views of one upload, or outputs of ``scb_locate_vortices``."""
+
+    nrhs: int
+    nv: int = 0
+    col_ptr: object = field(repr=False, default=None)  # torch int64 (nrhs + 1,)
+    nphi0: object = field(repr=False, default=None)    # torch f64 (nv,)
+    j_sub: object = field(repr=False, default=None)    # torch int64 (nv,)
+    j_all: object = field(repr=False, default=None)    # torch int64 (nv,)
+    row: object = field(repr=False, default=None)      # torch int64 (nv,)
+
+
+def make_vortex_state(film_info: FilmInfo, film_system: LinearSystem, columns) -> VortexState:
+    """``columns``: one sequence of ``Vortex`` per column of the solve (all in this film).  The table goes
+    to the device in one copy; the nearest vertices are found there (``scb_locate_vortices``), so the solve
+    needs no host synchronisation.  No device work when no column has a vortex."""
+    counts = [len(c) for c in columns]
+    nv = sum(counts)
+    if nv == 0:
+        return VortexState(nrhs=len(columns))
+    torch = _torch()
+    L = _lib.lib()
+    d = film_info.mesh._data
+    vortices = [v for c in columns for v in c]
+    col_ptr = np.zeros(len(columns) + 1, dtype=np.int64)
+    np.cumsum(counts, out=col_ptr[1:])
+    xy = np.array([(float(v.x), float(v.y)) for v in vortices], dtype=np.float64)
+    nphi0 = np.array([float(v.nPhi0) for v in vortices], dtype=np.float64)
+    # one host buffer (the float64 parts stored bit for bit as int64), one asynchronous copy from pinned
+    # memory: the caller's stream may still be factoring, and the host does not wait for it
+    host = torch.from_numpy(np.concatenate([col_ptr, xy.ravel().view(np.int64), nphi0.view(np.int64)]))
+    with torch.cuda.device(d.device):
+        buf = host.pin_memory().to(d.device, non_blocking=True)
+        nc = len(col_ptr)
+        col_ptr_d = buf[:nc]
+        xy_d = buf[nc:nc + 2 * nv].view(torch.float64)
+        nphi0_d = buf[nc + 2 * nv:].view(torch.float64)
+        j = torch.empty(2, nv, dtype=torch.int64, device=d.device)
+        _lib.check(L.scb_locate_vortices(nv, _lib.ptr(xy_d), d.n, _lib.ptr(d.sites), len(film_system.indices),
+                                         _lib.ptr(film_system.indices_dev), _lib.ptr(j[0]), _lib.ptr(j[1]),
+                                         _lib.stream_ptr()))
+        row = j[0]
+        if film_system.perm is not None:  # B[r] = h[perm[r]]: the vortex at system row j enters row invperm[j]
+            invperm = torch.empty_like(film_system.perm)
+            invperm[film_system.perm] = torch.arange(len(film_system.perm), dtype=torch.int64, device=d.device)
+            row = invperm[row]
+    return VortexState(nrhs=len(columns), nv=nv, col_ptr=col_ptr_d, nphi0=nphi0_d, j_sub=j[0], j_all=j[1], row=row)
+
+
+def apply_vortex_rhs(state: VortexState, film_info: FilmInfo, B, vortex_flux: float, scale=None,
+                     workspace: bool = True) -> None:
+    """Subtracts the vortex terms from the right-hand sides in place (``scb_vortex_rhs``): from the
+    triangular-solve workspace ``B`` (``workspace``: rows permuted and scaled as the factors need them), or
+    from ``h`` of ``(-A) x = h`` in system-row order (``lu_solve`` permutes and scales it)."""
+    L = _lib.lib()
+    d = film_info.mesh._data
+    assert B.is_contiguous() and (B.shape[1] if B.dim() == 2 else 1) == state.nrhs
+    _lib.check(L.scb_vortex_rhs(state.nrhs, _lib.ptr(state.col_ptr), _lib.ptr(state.row if workspace else state.j_sub),
+                                _lib.ptr(state.j_all), _lib.ptr(state.nphi0), _lib.ptr(d.t["vertex_areas"]),
+                                float(vortex_flux), _lib.ptr(scale if workspace else None), _lib.ptr(B),
+                                _lib.stream_ptr()))
+
+
 def solve_film_device(*, film_info: FilmInfo, film_system: LinearSystem, hole_systems: Dict[str, LinearSystem],
                       applied_field, vortex_flux: float, field_from_other_films=None,
                       check_inversion: bool = False, circulating_currents=None, terminal_systems=None,
                       device: Optional[Device] = None, hole_state=None, want_self_field: bool = True,
-                      terminal_currents=None, transport_state=None):
+                      terminal_currents=None, transport_state=None, vortex_state=None):
     """Device-side body of ``solve_film`` (reference solve_film.py:483-565): all arguments and
     results are device tensors in solver units.  ``want_self_field=False`` skips the screening mat-vec
     ``Q @ (w g)`` (an output only: the next Jacobi step needs ``J``, not the self field) and returns
@@ -435,8 +503,11 @@ def solve_film_device(*, film_info: FilmInfo, film_system: LinearSystem, hole_sy
     names to a float or to a ``(B,)`` tensor.  ``hole_state`` = ``hole_boundary_state(...)`` if the
     caller has it already.  For a film with transport terminals, ``terminal_currents`` (default:
     ``film_info.terminal_currents``) is one ``{terminal: current}`` dict, or a sequence of B of them for a
-    batch, and ``transport_state`` = ``terminal_transport_state(...)`` if the caller has it already.  Returns ``(g, J, self_field)`` with shapes ``(n,), (n, 2), (n,)`` or
-    ``(n, B), (n, B, 2), (n, B)``.
+    batch, and ``transport_state`` = ``terminal_transport_state(...)`` if the caller has it already.
+    ``vortex_state`` = ``make_vortex_state(...)`` gives every column its own vortices (default: the film's
+    vortices in every column); the vortex term is a correction to the right-hand side of each column
+    (include/scb.h, scb_vortex_rhs), so it costs no solve of its own.  Returns ``(g, J, self_field)`` with
+    shapes ``(n,), (n, 2), (n,)`` or ``(n, B), (n, B, 2), (n, B)``.
     """
     torch = _torch()
     L = _lib.lib()
@@ -447,6 +518,9 @@ def solve_film_device(*, film_info: FilmInfo, film_system: LinearSystem, hole_sy
     nrhs = applied_field.shape[1] if batched else 1
     transport = terminal_systems is not None
     with torch.cuda.device(d.device):
+        if vortex_state is None:
+            vortex_state = make_vortex_state(info, film_system, [info.vortices] * nrhs)
+        vortices = vortex_state.nv > 0
         if hole_state is None:
             hole_state = hole_boundary_state(info, hole_systems, circ, applied_field) if hole_systems \
                 else (None, None)
@@ -465,7 +539,7 @@ def solve_film_device(*, film_info: FilmInfo, film_system: LinearSystem, hole_sy
             s = _lib.stream_ptr()
             rhs_ix = film_system.indices_dev if film_system.rhs_indices_dev is None else film_system.rhs_indices_dev
             g = torch.empty_like(applied_c)
-            if not info.vortices:
+            if not vortices:
                 # right-hand side, triangular solves, stream function and current density in ONE foreign call
                 J = torch.empty((d.n, nrhs, 2) if batched else (d.n, 2), dtype=torch.float64, device=d.device)
                 _lib.check(L.scb_solve_step(
@@ -480,6 +554,7 @@ def solve_film_device(*, film_info: FilmInfo, film_system: LinearSystem, hole_sy
             _lib.check(L.scb_solve_rhs(n_int, n_pad, _lib.ptr(rhs_ix), nrhs, _lib.ptr(applied_c),
                                        _lib.ptr(other_c), _lib.ptr(Ha_eff), _lib.ptr(film_system.sym_scale),
                                        _lib.ptr(B), s))
+            apply_vortex_rhs(vortex_state, info, B, vortex_flux, scale=film_system.sym_scale)
             _lib.check(L.scb_getrs_nopiv(n_pad, _lib.ptr(film_system.lu), _lib.ptr(film_system.dinv), nrhs,
                                          _lib.ptr(B), s))
             _lib.check(L.scb_solve_stream(d.n, nrhs, _lib.ptr(film_system.pos), _lib.ptr(B),
@@ -501,6 +576,8 @@ def solve_film_device(*, film_info: FilmInfo, film_system: LinearSystem, hole_sy
                     Ha_eff = Ha_transport if Ha_eff is None else Ha_eff + Ha_transport
             ix = film_system.indices_dev
             h = Hz[ix] if Ha_eff is None else Hz[ix] - Ha_eff[ix]
+            if vortices:  # (the refinement and check_inversion residuals then see the true right-hand side)
+                apply_vortex_rhs(vortex_state, info, h, vortex_flux, workspace=False)
             gf = lu_solve(film_system, h)
             if film_system.refine or check_inversion:
                 # residual of (-A) gf = h through the matrix-free operator (reference check_inversion,
@@ -532,18 +609,6 @@ def solve_film_device(*, film_info: FilmInfo, film_system: LinearSystem, hole_sy
                         f"maximum error {r.abs().max().item():.3e} (relative {err:.3e})."
                     )
             g[ix] += gf
-        ix = film_system.indices_dev
-        for vortex in info.vortices:
-            # K[:, j] = -lu_solve(lu(-A), e_j): one right-hand side instead of eye(n)
-            # (reference solve_film.py:541-554)
-            xy = torch.tensor([vortex.x, vortex.y], dtype=torch.float64, device=d.device)
-            j_film = int(torch.argmin(torch.linalg.norm(d.sites[ix] - xy, dim=1)).item())
-            j_device = int(torch.argmin(torch.linalg.norm(d.sites - xy, dim=1)).item())
-            e = torch.zeros(len(film_system.indices), dtype=torch.float64, device=d.device)
-            e[j_film] = 1.0
-            Kj = -lu_solve(film_system, e)
-            gv = vortex_flux * vortex.nPhi0 * Kj / d.t["vertex_areas"][j_device]
-            g[ix] += gv[:, None] if batched else gv
         # J = curl(g z) = [dg/dy, -dg/dx]: (n, 2), or (n, B, 2) for a batch (source-major, the layout
         # of the film-to-film exchange)
         g = g.contiguous()
