@@ -10,7 +10,7 @@ from .device import Device, Layer, Polygon
 from .fluxoid import find_fluxoid_solution, make_fluxoid_polygons
 from .mesh import Mesh, MeshOperators
 from .meshgen import generate_mesh
-from .solution import FilmSolution, Fluxoid, Solution, Vortex
+from .solution import FilmSolution, Fluxoid, Solution, Vortex, field_at_position_batch
 from .solver import (
     FactorizedModel,
     FilmInfo,

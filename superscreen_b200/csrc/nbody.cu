@@ -60,11 +60,12 @@ struct NbodyParams {
 template <int KIND, int NR>
 struct Traits {
   static constexpr int tdim = (KIND == NB_Z || KIND == NB_VECTOR || KIND == NB_VECPOT) ? 3 : 2;
-  // NR = right-hand sides (NB_KERNEL), current-density sets sharing the geometry (film-to-film) or
+  // NR = right-hand sides (NB_KERNEL), current-density sets sharing the geometry (film-to-film, NB_Z) or
   // boundary stream sets sharing the edges (NB_BOUNDARY)
   static constexpr bool multi = KIND == NB_KERNEL || KIND == NB_FILM_TO_FILM || KIND == NB_COUPLING ||
-                                KIND == NB_BOUNDARY;
-  static constexpr int nacc = multi ? NR : (KIND == NB_VECTOR ? 4 : (KIND == NB_VECPOT || KIND == NB_Z ? 2 : 1));
+                                KIND == NB_BOUNDARY || KIND == NB_Z;
+  // NB_Z keeps two sums per set (Jx dy, Jy dx) and subtracts them only in nbody_store
+  static constexpr int nacc = KIND == NB_Z ? 2 * NR : (multi ? NR : (KIND == NB_VECTOR ? 4 : (KIND == NB_VECPOT ? 2 : 1)));
   static constexpr int npay = KIND == NB_KERNEL ? NR : (multi ? 2 * NR : 2);
   static constexpr bool has_sz = tdim == 3 || KIND == NB_COUPLING;
 };
@@ -83,7 +84,8 @@ __device__ __forceinline__ void nbody_store(const NbodyParams& p, int64_t i, con
 #pragma unroll
     for (int r = 0; r < NR; r++) p.out[i * p.ldo + p.rhs0 + r] = pf * acc[r];
   } else if (KIND == NB_Z) {
-    p.out[i] = pf * (acc[0] - acc[1]);
+#pragma unroll
+    for (int r = 0; r < NR; r++) p.out[r * p.m + i] = pf * (acc[2 * r] - acc[2 * r + 1]);
   } else if (KIND == NB_VECTOR) {
     p.out[3 * i] = pf * acc[3];
     p.out[3 * i + 1] = -(pf * acc[2]);
@@ -152,7 +154,7 @@ __global__ void __launch_bounds__(256) nbody_kernel(NbodyParams p) {
         if (KIND == NB_KERNEL) {
 #pragma unroll
           for (int r = 0; r < NR; r++) spay[r][tid] = p.J ? w * p.J[js * p.ldv + p.rhs0 + r] : w;
-        } else if (KIND == NB_FILM_TO_FILM) {
+        } else if (KIND == NB_FILM_TO_FILM || KIND == NB_Z) {
 #pragma unroll
           for (int r = 0; r < NR; r++) {
             spay[2 * r][tid] = w * p.J[(r * p.n + js) * 2];
@@ -211,8 +213,11 @@ __global__ void __launch_bounds__(256) nbody_kernel(NbodyParams p) {
 #pragma unroll
             for (int r = 0; r < NR; r++) acc[k][r] = fma(-k3, fma(pay[2 * r], dx, pay[2 * r + 1] * dy), acc[k][r]);
           } else if (KIND == NB_Z) {
-            acc[k][0] = fma(k3 * pay[0], dy, acc[k][0]);  // Jx_dy
-            acc[k][1] = fma(k3 * pay[1], dx, acc[k][1]);  // Jy_dx
+#pragma unroll
+            for (int r = 0; r < NR; r++) {
+              acc[k][2 * r] = fma(k3 * pay[2 * r], dy, acc[k][2 * r]);              // Jx_dy
+              acc[k][2 * r + 1] = fma(k3 * pay[2 * r + 1], dx, acc[k][2 * r + 1]);  // Jy_dx
+            }
           } else {                                        // NB_VECTOR
             const double px = k3 * pay[0], py = k3 * pay[1];
             acc[k][0] = fma(px, dy, acc[k][0]);   // Jx_dy
@@ -276,11 +281,14 @@ static int launch_nbody(NbodyParams p, cudaStream_t s) {
   const int64_t ctas_x = ceil_div(p.m, 256 * TPT);
   // One balanced wave: every CTA does the same amount of work, so the source range is split until the
   // grid just fills the resident-CTA capacity of the device (a CTA keeps at least one source tile).
+  // NB_Z passes of several sets split as the single-set pass does, whatever their own occupancy: the
+  // split fixes the summation order, so every set of a multi-set call has the bits of a one-set call.
+  constexpr int CAP_NR = KIND == NB_Z ? 1 : NR;
   static int capacity = 0;  // per instantiation; all devices of a node are identical
   if (capacity == 0) {
     int per_sm = 0, sms = 0, dev = 0;
     SCB_CUDA(cudaGetDevice(&dev));
-    SCB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, nbody_kernel<KIND, NR>, 256, 0));
+    SCB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, nbody_kernel<KIND, CAP_NR>, 256, 0));
     SCB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     capacity = per_sm * sms > 0 ? per_sm * sms : 148;
   }
@@ -640,7 +648,12 @@ extern "C" int scb_biot_savart(int kind, int64_t m, const double* tgt, int64_t n
         else if (nsets - k >= 2) { rc = launch_nbody<NB_FILM_TO_FILM, 2>(p, s); step = 2; }
         else rc = launch_nbody<NB_FILM_TO_FILM, 1>(p, s);
         break;
-      case SCB_BS_Z: rc = launch_nbody<NB_Z, 1>(p, s); break;
+      case SCB_BS_Z:  // as film-to-film: one r^-3 per pair serves every set of a pass
+        if (nsets - k >= 8) { rc = launch_nbody<NB_Z, 8>(p, s); step = 8; }
+        else if (nsets - k >= 4) { rc = launch_nbody<NB_Z, 4>(p, s); step = 4; }
+        else if (nsets - k >= 2) { rc = launch_nbody<NB_Z, 2>(p, s); step = 2; }
+        else rc = launch_nbody<NB_Z, 1>(p, s);
+        break;
       case SCB_BS_VECTOR: rc = launch_nbody<NB_VECTOR, 1>(p, s); break;
       case SCB_BS_VECTOR_POTENTIAL: rc = launch_nbody<NB_VECPOT, 1>(p, s); break;
       default: set_error("scb_biot_savart: unknown kind %d", kind); return SCB_ERR_INVALID;

@@ -691,19 +691,273 @@ class Solution:
         return out
 
 
+class _FilmBatch(NamedTuple):
+    """One film's share of a staged ``field_at_position_batch``."""
+
+    name: str
+    src: np.ndarray                # (n, 3) vertices and layer height, meters
+    areas: np.ndarray              # (n,) vertex areas, square meters
+    J: Any                         # pinned (B, n, 2) current densities, A / m
+    out_idx: Optional[np.ndarray]  # positions evaluated by the pair sum (None: all of them)
+    in_idx: Optional[np.ndarray]   # positions inside the film, in its plane
+    in_field: Optional[np.ndarray]  # (B, len(in_idx)) interpolated self field there, tesla
+
+
+class _FieldBatchStage(NamedTuple):
+    """Host side of ``field_at_position_batch``: checked inputs and staged arrays, no device work."""
+
+    B: int
+    m: int
+    targets: Any                   # pinned (m, 3) evaluation points, meters
+    films: List[_FilmBatch]
+    to_field_units: float          # tesla -> field_units
+    to_units: float                # field_units -> units
+    units: str
+    applied: np.ndarray            # (k, m) distinct applied-field rows, in units
+    applied_row: np.ndarray        # (B,) row of ``applied`` of every entry
+
+
+def _interp_batch(mesh, rows: Sequence[Optional[np.ndarray]], xy: np.ndarray) -> np.ndarray:
+    """``interp_field`` of B datasets on one mesh at the same points (the triangles are located once): (B, q),
+    zero outside the mesh and where the value is not finite."""
+    out = np.zeros((len(rows), len(xy)))
+    if len(xy) == 0:
+        return out
+    ok, tri, w = _locate(mesh.sites, mesh.elements, xy, 16)
+    for b, values in enumerate(rows):  # (a missing dataset, such as field_from_other_films of one film, is zero)
+        if values is not None:
+            out[b] = np.einsum("qk,qk->q", w, np.asarray(values, dtype=float)[mesh.elements[tri]])
+    out[:, ~ok] = 0
+    out[~np.isfinite(out)] = 0
+    return out
+
+
+def _stage_field_batch(solutions, positions, zs, interp_method: str, units: Optional[str]) -> _FieldBatchStage:
+    import torch
+
+    solutions = list(solutions)
+    for b, sol in enumerate(solutions):
+        if not isinstance(sol, Solution):
+            raise TypeError(f"solutions[{b}] is a {type(sol).__name__}, not a Solution.")
+    positions, zs = _normalize_positions(positions, zs, np.float64)
+    B, m = len(solutions), len(positions)
+    if B == 0:
+        return _FieldBatchStage(0, m, None, [], 1.0, 1.0, units, np.zeros((0, m)), np.zeros(0, dtype=np.int64))
+    first = solutions[0]
+    device = first.device
+    film_names = list(device.films)
+    for b, sol in enumerate(solutions):
+        d = sol.device
+        if list(d.films) != film_names:
+            raise ValueError(f"solutions[{b}] has the films {list(d.films)}, solutions[0] has {film_names}.")
+        if d.length_units != device.length_units:
+            raise ValueError(f"solutions[{b}] has length_units {d.length_units!r}, solutions[0] has "
+                             f"{device.length_units!r}.")
+        if sol.field_units != first.field_units or sol.current_units != first.current_units:
+            raise ValueError(f"solutions[{b}] has units ({sol.field_units!r}, {sol.current_units!r}), solutions[0] "
+                             f"has ({first.field_units!r}, {first.current_units!r}).")
+        for name in film_names:
+            if name not in sol.film_solutions:
+                raise ValueError(f"solutions[{b}] holds no solution of film {name!r} (a solve_batch(gather=False) "
+                                 f"result holds only the films of its rank).")
+            mesh, mesh0 = d.meshes[name], device.meshes[name]
+            if mesh is not mesh0 and not (np.array_equal(mesh.sites, mesh0.sites)
+                                          and np.array_equal(mesh.elements, mesh0.elements)):
+                raise ValueError(f"solutions[{b}] has another mesh of film {name!r} than solutions[0].")
+            z0, z0_first = d.layers[d.films[name].layer].z0, device.layers[device.films[name].layer].z0
+            if z0 != z0_first:
+                raise ValueError(f"solutions[{b}] has film {name!r} at z0 = {z0}, solutions[0] at z0 = {z0_first}.")
+    in_plane = [np.all(zs == device.layers[film.layer].z0) for film in device.films.values()]
+    if interp_method != "linear" and any(in_plane):  # (as interp_field raises it)
+        raise NotImplementedError("Only linear interpolation is available.")
+
+    field_units, current_units, length_units = first.field_units, first.current_units, device.length_units
+    units = units or field_units
+    to_meter = _u.conversion_factor(length_units, "m")
+    to_amp_per_meter = _u.conversion_factor(f"({current_units}) / ({length_units})", "A / m")
+    # (the same host arithmetic as biot_savart_2d, so the device sees the same operands)
+    targets = torch.empty((m, 3), dtype=torch.float64, pin_memory=True)
+    ev = targets.numpy()
+    np.multiply(positions[:, 0], to_meter, out=ev[:, 0])
+    np.multiply(positions[:, 1], to_meter, out=ev[:, 1])
+    np.multiply(np.broadcast_to(zs, (m,)), to_meter, out=ev[:, 2])
+    films = []
+    for (name, film), plane in zip(device.films.items(), in_plane):
+        mesh = device.meshes[name]
+        z0 = device.layers[film.layer].z0
+        out_idx = in_idx = in_field = None
+        if plane:
+            in_film = film.contains_points(positions)
+            in_idx, out_idx = np.flatnonzero(in_film), np.flatnonzero(~in_film)
+            in_field = _interp_batch(mesh, [s.film_solutions[name].self_field for s in solutions], positions[in_idx])
+            if field_units != "tesla":
+                from .solver.utils import convert_field
+
+                in_field = convert_field(in_field, "tesla", old_units=field_units, with_units=False)
+            if len(out_idx) == m:
+                out_idx = in_idx = in_field = None
+        n = len(mesh.sites)
+        src = np.ascontiguousarray(np.concatenate([mesh.sites * to_meter, (z0 * np.ones(n) * to_meter)[:, None]],
+                                                  axis=1), dtype=np.float64)
+        areas = np.ascontiguousarray(np.asarray(mesh.vertex_areas) * to_meter**2, dtype=np.float64)
+        J = torch.empty((B, n, 2), dtype=torch.float64, pin_memory=True)
+        Jh = J.numpy()
+        for b, sol in enumerate(solutions):
+            Jh[b] = np.atleast_2d(sol.film_solutions[name].current_density) * to_amp_per_meter
+        films.append(_FilmBatch(name, src, areas, J, out_idx, in_idx, in_field))
+
+    # applied field (field_at_position): interpolated from the solutions at in-plane points inside a film, the
+    # applied-field function elsewhere -- evaluated once per distinct function object
+    in_film = np.zeros(m, dtype=bool)
+    per_entry = None
+    films_by_layer = device.polygons_by_layer("film")
+    for lname, layer in device.layers.items():
+        if np.all(zs == layer.z0):
+            per_entry = np.zeros((B, m))
+            for film in films_by_layer[lname]:
+                ix = film.contains_points(positions)
+                in_film[ix] = True
+                mesh, xy = device.meshes[film.name], positions[ix]
+                fss = [s.film_solutions[film.name] for s in solutions]
+                per_entry[:, ix] = (_interp_batch(mesh, [fs.applied_field for fs in fss], xy)
+                                    + _interp_batch(mesh, [fs.field_from_other_films for fs in fss], xy))
+            break
+    mask = ~in_film
+    func_row: Dict[int, int] = {}
+    rows = []
+    applied_row = np.empty(B, dtype=np.int64)
+    for b, sol in enumerate(solutions):
+        func = sol.applied_field_func
+        k = func_row.get(id(func))
+        if k is None and mask.any():
+            value = np.squeeze(func(positions[mask, 0], positions[mask, 1], zs[mask, np.newaxis]))
+            rows.append(np.broadcast_to(np.asarray(value, dtype=np.float64), (int(mask.sum()),)))
+        if k is None:
+            k = func_row[id(func)] = len(func_row)
+        applied_row[b] = k
+    if per_entry is None:
+        applied = np.stack(rows) if rows else np.zeros((len(func_row), m))
+    else:
+        if mask.any():
+            for b in range(B):
+                per_entry[b, mask] = rows[applied_row[b]]
+        applied, applied_row = per_entry, np.arange(B)
+    to_units = _field_factor(field_units, units)
+    if to_units != 1.0:
+        applied = applied * to_units
+    return _FieldBatchStage(B, m, targets, films, _field_factor("tesla", field_units), to_units, units,
+                            applied, applied_row)
+
+
+def _evaluate_field_batch(stage: _FieldBatchStage, return_sum: bool):
+    """Device side of ``field_at_position_batch``: one multi-set pair sum per film and chunk of targets, the unit
+    factors and the sum over films on the device, one copy of every result to the host."""
+    import torch
+
+    L = _lib.lib()
+    B, m = stage.B, stage.m
+    dev = torch.device(f"cuda:{torch.cuda.current_device()}")
+    with torch.cuda.device(dev):
+        targets = stage.targets.to(dev, non_blocking=True)
+        total, fields = None, {}
+        for f in stage.films:
+            src, areas, J = (torch.as_tensor(a).to(dev, non_blocking=True) for a in (f.src, f.areas, f.J))
+            field = torch.empty((B, m), dtype=torch.float64, device=dev)
+            if f.out_idx is None:
+                tgt = targets
+            else:
+                out_idx = torch.as_tensor(f.out_idx).to(dev)
+                tgt = targets.index_select(0, out_idx)
+                field[:, torch.as_tensor(f.in_idx).to(dev)] = torch.as_tensor(f.in_field).to(dev)
+            # the chunks of biot_savart_2d: the source split of the pair sum, hence every bit of it, depends on
+            # the number of targets of a launch
+            mf = int(tgt.shape[0])
+            chunk = mf if mf <= _EVAL_CHUNK else _EVAL_CHUNK
+            for lo in range(0, mf, max(chunk, 1)):
+                hi = min(mf, lo + chunk)
+                direct = f.out_idx is None and hi - lo == m
+                out = field if direct else torch.empty((B, hi - lo), dtype=torch.float64, device=dev)
+                _lib.check(L.scb_biot_savart(1, hi - lo, _lib.ptr(tgt[lo:hi]), int(src.shape[0]), _lib.ptr(src),
+                                             _lib.ptr(areas), _lib.ptr(J), 0.0, _MU0_BIOT_SAVART / (4 * np.pi), B,
+                                             _lib.ptr(out), _lib.stream_ptr()))
+                if f.out_idx is not None:
+                    field[:, out_idx[lo:hi]] = out
+                elif not direct:
+                    field[:, lo:hi] = out
+            # tesla -> field_units -> units, then films in device order: the operations of field_at_position
+            if stage.to_field_units != 1.0:
+                field.mul_(stage.to_field_units)
+            if stage.to_units != 1.0:
+                field.mul_(stage.to_units)
+            if not return_sum:
+                fields[f.name] = field
+            elif total is None:
+                total = field
+            else:
+                total.add_(field)
+        results = fields
+        if return_sum:
+            applied = torch.as_tensor(stage.applied).to(dev).index_select(0, torch.as_tensor(stage.applied_row).to(dev))
+            if total is None:
+                total = applied
+            else:
+                total.add_(applied)
+            results = {"total": total}
+        host = {}
+        for key, t in results.items():
+            host[key] = torch.empty((B, m), dtype=torch.float64, pin_memory=True)
+            host[key].copy_(t, non_blocking=True)
+        torch.cuda.current_stream(dev).synchronize()
+    if return_sum:
+        return host["total"].numpy()
+    out = {key: t.numpy() for key, t in host.items()}
+    out["applied_field"] = stage.applied[stage.applied_row]
+    return out
+
+
+def field_at_position_batch(solutions: Sequence["Solution"], positions, *, zs=None, interp_method: str = "linear",
+                            units: Optional[str] = None, with_units: bool = True, return_sum: bool = True):
+    """``Solution.field_at_position`` of B solutions of one device (e.g. the entries of a ``solve_batch``) at the
+    same positions, in one pass: row ``b`` is ``solutions[b].field_at_position(positions, zs=zs,
+    interp_method=interp_method, units=units, with_units=False, return_sum=return_sum)``.
+
+    Returns a ``(B, m)`` array (a ``Quantity`` with ``with_units``), or with ``return_sum=False`` a dict of
+    ``(B, m)`` arrays, one per film and ``"applied_field"``.  Every film's field at the points off its plane is one
+    pair sum over all B current densities (one r^-3 per pair serves the B entries), and its bits are those of the
+    per-solution call.  The solutions must share the films, their meshes and heights, the length units, the field
+    units and the current units; each must hold every film.  Applied-field functions are evaluated once per
+    distinct function object."""
+    stage = _stage_field_batch(solutions, positions, zs, interp_method, units)
+    if stage.B == 0:
+        value = np.empty((0, stage.m)) if return_sum else {}
+    else:
+        value = _evaluate_field_batch(stage, return_sum)
+    if not with_units or (stage.B == 0 and units is None):
+        return value
+    if return_sum:
+        return _u.Quantity(value, stage.units)
+    return {key: _u.Quantity(v, stage.units) for key, v in value.items()}
+
+
 _FIELD_FACTORS: Dict[tuple, float] = {}
 
 
-def _convert_owned(value, new_units: str, old_units: str, with_units: bool, owned: bool = True):
-    """``convert_field`` for an array this module has just produced itself (a million-point field evaluation
-    makes half a dozen such passes): the factor is looked up once per unit pair, a factor of one costs nothing
-    and the scaling is done in place."""
+def _field_factor(old_units: str, new_units: str) -> float:
+    """The ``convert_field`` factor from ``old_units`` to ``new_units``, looked up once per unit pair."""
     from .solver.utils import convert_field
 
     key = (str(old_units), str(new_units))
     factor = _FIELD_FACTORS.get(key)
     if factor is None:
         factor = _FIELD_FACTORS[key] = float(convert_field(1.0, new_units, old_units=old_units, with_units=False))
+    return factor
+
+
+def _convert_owned(value, new_units: str, old_units: str, with_units: bool, owned: bool = True):
+    """``convert_field`` for an array this module has just produced itself (a million-point field evaluation
+    makes half a dozen such passes): the factor is looked up once per unit pair, a factor of one costs nothing
+    and the scaling is done in place."""
+    factor = _field_factor(old_units, new_units)
     if factor != 1.0:
         if owned and isinstance(value, np.ndarray) and value.flags.writeable and value.dtype == np.float64:
             np.multiply(value, factor, out=value)
