@@ -138,6 +138,62 @@ int scb_delaunay(int64_t n, const double* points, double x0, double y0, double c
                  int64_t max_triangles, int64_t* triangles, int64_t* info, scb_stream_t stream);
 
 /* ------------------------------------------------------------------------------------
+ * Point location and linear interpolation on a triangulation, polygon masks: the device stage of
+ * Solution.interp_current_density / interp_field for a batch of solutions (solution.py:272-276,310-312,
+ * which stand in for matplotlib's LinearTriInterpolator; geometry.points_in_polygon, geometry.py:77-103).
+ * ------------------------------------------------------------------------------------ */
+
+/* int32 workspace elements of scb_tri_grid_count / _fill for ntri triangles and ncells = ncx * ncy cells.
+ * Layout: per-triangle cell ranges [4 ntri] | start [ncells + 1] | fill [ncells]; 16-byte aligned. */
+int64_t scb_tri_grid_workspace_elems(int64_t ntri, int64_t ncells);
+
+/* Uniform cell grid over the triangles of a mesh: cell (i, j) = [x0 + i cell, x0 + (i + 1) cell) x [y0 + j cell,
+ * ...), i < ncx, j < ncy.  Every triangle is registered in every cell that its bounding box overlaps, the box
+ * padded so that no point whose rounded barycentric coordinates (scb_tri_locate) are all >= -1e-12 falls outside
+ * it; an all but degenerate triangle (longest edge^2 / |det| >= 2^-8 / eps) is registered in every cell, one with
+ * det == 0 in none.  Two calls with a host read in between:
+ *   scb_tri_grid_count  cell ranges and counts, exclusive scan: workspace[4 ntri + ncells] <- number of entries;
+ *   scb_tri_grid_fill   cell_tris (int32 [entries]) <- the triangles of every cell, cell after cell (cell c:
+ *                       cell_tris[start[c] .. start[c + 1]), start = workspace + 4 ntri), ascending per cell. */
+int scb_tri_grid_count(int64_t ntri, const double* sites, const int64_t* elements, double x0, double y0, double cell,
+                       int32_t ncx, int32_t ncy, int32_t* workspace, scb_stream_t stream);
+int scb_tri_grid_fill(int64_t ntri, int32_t ncx, int32_t ncy, int32_t* workspace, int32_t* cell_tris,
+                      scb_stream_t stream);
+
+/* Containing triangle of q points xy [q, 2]: tri (int64 [q], -1 outside) and bary (f64 [q, 3]; 0 outside).  The
+ * result is a function of the mesh and the grid bounds alone; the grid only prunes the candidates:
+ *  - the barycentric coordinates are _barycentric's (solution.py:122-130) operation by operation, one rounding
+ *    per operation, no FMA contraction, l3 = (1.0 - l1) - l2;
+ *  - the point's triangle is the one, among all triangles, with the largest min(l1, l2, l3), ties to the lowest
+ *    index; a triangle with a non-finite coordinate never wins;
+ *  - the point is inside iff that maximum is >= -1e-12;
+ *  - a point with a non-finite coordinate, or outside [x0, x1] x [y0, y1] (x1 = x0 + ncx cell and y1 = y0 +
+ *    ncy cell as the caller computed them), is outside.
+ * The order of the cell lists does not matter.  start / cell_tris are those of scb_tri_grid_fill. */
+int scb_tri_locate(int64_t q, const double* xy, const double* sites, const int64_t* elements, double x0, double y0,
+                   double x1, double y1, double cell, int32_t ncx, int32_t ncy, const int32_t* start,
+                   const int32_t* cell_tris, int64_t* tri, double* bary, scb_stream_t stream);
+
+/* Linear interpolation of nsets value sets at q located points: values [nsets, n, ncomp] (set-major, as a batch
+ * is staged: one contiguous copy of the B arrays; the output is set-major too, so the writes of a warp are
+ * contiguous), ncomp 1 or 2, out [nsets, q, ncomp]:
+ *   out[s, p, c] = (0.0 + sum) * scale,  sum over the corners k of w_k v_k (one rounding per operation) in the
+ *   order of np.einsum("qk,qk...->q...") (measured on the host): ncomp = 1: (w0 v0 + w2 v2) + w1 v1;
+ *   ncomp = 2: (w0 v0 + w1 v1) + w2 v2; the 0.0 + of einsum's accumulator turns -0.0 into +0.0.
+ * out is 0 where tri < 0, where mask (uint8 [q], may be NULL) is 0, and for every component of a point whose
+ * components are not all finite. */
+int scb_tri_interpolate(int64_t q, const int64_t* tri, const double* bary, const int64_t* elements, int64_t nsets,
+                        int ncomp, int64_t n, const double* values, const uint8_t* mask, double scale, double* out,
+                        scb_stream_t stream);
+
+/* Even-odd test of m points against ONE ring of nv vertices (open: the closing edge is implicit), bit for bit
+ * geometry.points_in_polygon: edges half-open in y, crossing abscissa dx * (y - y1) / dy + x1 rounded in that
+ * order.  op 0: inside = test; 1: inside |= test; 2: inside &= !test (the rings of a CompositePolygon,
+ * device.py:286-293).  Not scb_points_in_rings, which rounds in another order. */
+int scb_points_in_polygon(int64_t m, const double* points, int64_t nv, const double* vertices, int op,
+                          uint8_t* inside, scb_stream_t stream);
+
+/* ------------------------------------------------------------------------------------
  * Kernel matrix pieces and system assembly  (K1-K3, K8-K10, K19, rows a1-a3, a9-a11)
  *   distance.py:87-115 q_matrix, device/mesh.py:434-458 Q_matrix,
  *   solver/utils.py:290-297 (dense casts, never materialised here),

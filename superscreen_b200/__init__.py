@@ -5,12 +5,13 @@ Public names mirror ``superscreen/__init__.py:1-20`` for the path in scope (SURV
 ``Vortex``, ``Device``, ``Layer``, ``Polygon``, ``Mesh``, ``fem``, ``distance``, ``sources``.
 All arithmetic runs in ``libsc_b200.so`` (include/scb.h); there is no CPU fallback.
 """
-from . import distance, fem, geometry, io, meshgen, parallel, sources, units
+from . import distance, fem, geometry, interp, io, meshgen, parallel, sources, units
 from .device import Device, Layer, Polygon
 from .fluxoid import find_fluxoid_solution, make_fluxoid_polygons
 from .mesh import Mesh, MeshOperators
 from .meshgen import generate_mesh
-from .solution import FilmSolution, Fluxoid, Solution, Vortex, field_at_position_batch
+from .solution import (FilmSolution, Fluxoid, Solution, Vortex, field_at_position_batch, interp_current_density_batch,
+                       interp_field_batch)
 from .solver import (
     FactorizedModel,
     FilmInfo,

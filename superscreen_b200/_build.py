@@ -11,7 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libsc_b200.so")
 SOURCES = ["api.cu", "mesh_ops.cu", "nbody.cu", "assemble.cu", "getrf.cu", "getrs.cu", "spmv.cu", "diag.cu", "delaunay.cu",
-           "vortex.cu"]
+           "vortex.cu", "interp.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xptxas=-v",
@@ -26,7 +26,7 @@ def _nvcc() -> str:
 
 
 STAMP = LIB + ".stamp"
-ABI_VERSION = 203  # must equal scb_version() of the sources (csrc/api.cu)
+ABI_VERSION = 204  # must equal scb_version() of the sources (csrc/api.cu)
 
 
 def source_digest() -> str:

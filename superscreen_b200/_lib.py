@@ -76,6 +76,15 @@ EXPORTS = {
                                    c_void_p, c_int64, c_void_p, c_double, c_void_p, c_void_p, c_void_p]),
     "scb_delaunay": (c_int, [c_int64, c_void_p, c_double, c_double, c_double, c_int32, c_int32, c_int64, c_void_p,
                              c_void_p, c_void_p]),
+    "scb_tri_grid_workspace_elems": (c_int64, [c_int64, c_int64]),
+    "scb_tri_grid_count": (c_int, [c_int64, c_void_p, c_void_p, c_double, c_double, c_double, c_int32, c_int32, c_void_p,
+                                   c_void_p]),
+    "scb_tri_grid_fill": (c_int, [c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p]),
+    "scb_tri_locate": (c_int, [c_int64, c_void_p, c_void_p, c_void_p, c_double, c_double, c_double, c_double, c_double,
+                               c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "scb_tri_interpolate": (c_int, [c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int64, c_void_p, c_void_p,
+                                    c_double, c_void_p, c_void_p]),
+    "scb_points_in_polygon": (c_int, [c_int64, c_void_p, c_int64, c_void_p, c_int, c_void_p, c_void_p]),
 }
 
 

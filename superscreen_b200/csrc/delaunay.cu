@@ -352,6 +352,18 @@ __global__ void delaunay_info_kernel(int64_t n, const int32_t* __restrict__ offs
   }
 }
 
+// the scan and the per-cell sort for other cell grids (interp.cu's triangle grid)
+int launch_cell_scan(int32_t* count, int64_t ncells, cudaStream_t s) {
+  scan_kernel<<<1, 1024, 0, s>>>(count, ncells);
+  SCB_LAUNCH_CHECK();
+  return SCB_OK;
+}
+int launch_cell_sort(int64_t ncells, const int32_t* start, int32_t* order, cudaStream_t s) {
+  cell_sort_kernel<<<(unsigned)ceil_div(ncells, 256), 256, 0, s>>>(ncells, start, order);
+  SCB_LAUNCH_CHECK();
+  return SCB_OK;
+}
+
 }  // namespace scb
 
 using namespace scb;

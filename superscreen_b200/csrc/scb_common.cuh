@@ -39,6 +39,11 @@ void count_launch(int n = 1);
     }                                                                               \
   } while (0)
 
+// delaunay.cu: exclusive scan of count[0 .. ncells) in place with the total in count[ncells] (one CTA), and the
+// sort of every cell's list order[start[c] .. start[c + 1]) by value
+int launch_cell_scan(int32_t* count, int64_t ncells, cudaStream_t s);
+int launch_cell_sort(int64_t ncells, const int32_t* start, int32_t* order, cudaStream_t s);
+
 static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
 constexpr double kOneOver4Pi = 0.07957747154594767;  // 1/(4*pi)

@@ -939,6 +939,149 @@ def field_at_position_batch(solutions: Sequence["Solution"], positions, *, zs=No
     return {key: _u.Quantity(v, stage.units) for key, v in value.items()}
 
 
+# interpolated values per chunk of targets (B * points * components): bounds the device output buffer to 512 MiB
+_INTERP_CHUNK_ELEMS = 1 << 26
+
+
+def _stage_interp_batch(solutions, positions, film: str, method: str):
+    """Host checks of the interpolation batches: (solutions, positions (m, 2)); raises before any device work."""
+    solutions = list(solutions)
+    for b, sol in enumerate(solutions):
+        if not isinstance(sol, Solution):
+            raise TypeError(f"solutions[{b}] is a {type(sol).__name__}, not a Solution.")
+    if method != "linear":
+        raise NotImplementedError("Only linear interpolation is available.")
+    positions = np.ascontiguousarray(np.atleast_2d(np.asarray(positions, dtype=np.float64))[:, :2])
+    if not solutions:
+        return solutions, positions
+    first = solutions[0]
+    for b, sol in enumerate(solutions):
+        d = sol.device
+        if film not in d.films:
+            raise ValueError(f"solutions[{b}] has no film {film!r} (films: {list(d.films)}).")
+        if film not in sol.film_solutions:
+            raise ValueError(f"solutions[{b}] holds no solution of film {film!r} (a solve_batch(gather=False) "
+                             f"result holds only the films of its rank).")
+        mesh, mesh0 = d.meshes[film], first.device.meshes[film]
+        if mesh is not mesh0 and not (np.array_equal(mesh.sites, mesh0.sites)
+                                      and np.array_equal(mesh.elements, mesh0.elements)):
+            raise ValueError(f"solutions[{b}] has another mesh of film {film!r} than solutions[0].")
+        if (sol.field_units, sol.current_units, d.length_units) != (first.field_units, first.current_units,
+                                                                    first.device.length_units):
+            raise ValueError(f"solutions[{b}] has units ({sol.field_units!r}, {sol.current_units!r}, "
+                             f"{d.length_units!r}), solutions[0] has ({first.field_units!r}, "
+                             f"{first.current_units!r}, {first.device.length_units!r}).")
+    return solutions, positions
+
+
+def _interp_batch_device(mesh, rows: Sequence[Optional[np.ndarray]], ncomp: int, positions: np.ndarray, polygon,
+                         scale: float) -> np.ndarray:
+    """Device side of the interpolation batches: (B, m, ncomp) values of the B value sets ``rows`` (None: zeros)
+    at ``positions``.  The targets run in chunks of ``_INTERP_CHUNK_ELEMS // (B ncomp)`` points: each chunk is
+    located and masked once for all B sets; the device holds the mesh, its grid, the B value sets, the positions
+    and one chunk of results; every chunk is copied back behind its kernels, one synchronisation at the end."""
+    import torch
+
+    from . import interp
+
+    B, m = len(rows), len(positions)
+    n = len(mesh.sites)
+    dev = torch.device(f"cuda:{torch.cuda.current_device()}")
+    with torch.cuda.device(dev):
+        grid = interp.tri_grid(mesh.sites, mesh.elements)
+        vals = torch.empty((B, n, ncomp), dtype=torch.float64, pin_memory=True)
+        vh = vals.numpy()
+        for b, v in enumerate(rows):
+            if v is None:
+                vh[b] = 0.0
+            else:
+                vh[b] = np.asarray(v, dtype=np.float64).reshape(n, ncomp)
+        pos_pin = torch.empty((m, 2), dtype=torch.float64, pin_memory=True)
+        pos_pin.numpy()[:] = positions
+        vals_d = vals.to(dev, non_blocking=True)
+        xy_d = pos_pin.to(dev, non_blocking=True)
+        rings = interp.upload_rings(polygon, dev) if polygon is not None else None
+        host = torch.empty((B, m, ncomp), dtype=torch.float64, pin_memory=True)
+        chunk = max(1, min(m, _INTERP_CHUNK_ELEMS // max(B * ncomp, 1)))
+        # one set of chunk buffers: every use is ordered on this stream behind the copy of the previous chunk
+        tri = torch.empty(chunk, dtype=torch.int64, device=dev)
+        bary = torch.empty((chunk, 3), dtype=torch.float64, device=dev)
+        inside = torch.empty(chunk, dtype=torch.uint8, device=dev) if rings is not None else None
+        out = torch.empty((B, chunk, ncomp), dtype=torch.float64, device=dev)
+        for lo in range(0, m, chunk):
+            hi = min(m, lo + chunk)
+            c = hi - lo
+            xy = xy_d[lo:hi]
+            interp.locate(grid, xy, tri[:c], bary[:c])
+            if rings is not None:
+                interp.polygon_mask(rings, xy, inside[:c])
+            o = out if c == chunk else torch.empty((B, c, ncomp), dtype=torch.float64, device=dev)
+            interp.interpolate(grid, tri[:c], bary[:c], vals_d, o, None if inside is None else inside[:c], scale)
+            if c == m:
+                host.copy_(o, non_blocking=True)
+            else:
+                for b in range(B):
+                    host[b, lo:hi].copy_(o[b], non_blocking=True)
+        torch.cuda.current_stream(dev).synchronize()
+    return host.numpy()
+
+
+def interp_current_density_batch(solutions: Sequence["Solution"], positions, *, film: str, method: str = "linear",
+                                 units: Optional[str] = None, with_units: bool = False):
+    """``Solution.interp_current_density`` of B solutions of one device at the same positions, on the GPU: a
+    ``(B, m, 2)`` array whose row ``b`` is ``solutions[b].interp_current_density(positions, film=film,
+    method=method, units=units, with_units=False)`` (a ``Quantity`` with ``with_units``).
+
+    The positions are located in the film's mesh once for all entries (the triangle with the largest smallest
+    barycentric coordinate, scb_tri_locate) and masked by the film polygon once; where the host and the device
+    choose the same triangle the values carry the host's bits.  The solutions must share the film's mesh and
+    their units, and each must hold the film.  Only ``method="linear"`` is available."""
+    solutions, positions = _stage_interp_batch(solutions, positions, film, method)
+    m = len(positions)
+    if not solutions:
+        J = np.zeros((0, m, 2))
+        return _u.Quantity(J, units) if with_units and units is not None else J
+    first = solutions[0]
+    device = first.device
+    default_units = f"({first.current_units}) / ({device.length_units})"
+    scale = 1.0
+    if units is not None and units != default_units:
+        scale = _u.conversion_factor(default_units, units)
+    J = np.zeros((len(solutions), m, 2))
+    if m:
+        J = _interp_batch_device(device.meshes[film], [s.film_solutions[film].current_density for s in solutions], 2,
+                                 positions, device.films[film], scale)
+    return _u.Quantity(J, units or default_units) if with_units else J
+
+
+def interp_field_batch(solutions: Sequence["Solution"], positions, *, film: str, dataset: str = "total_field",
+                       method: str = "linear", units: Optional[str] = None, with_units: bool = False):
+    """``Solution.interp_field`` of B solutions of one device at the same positions, on the GPU: a ``(B, m)`` array
+    whose row ``b`` is ``solutions[b].interp_field(positions, film=film, dataset=dataset, method=method,
+    units=units, with_units=False)`` (a ``Quantity`` with ``with_units``).  A dataset that is None (e.g.
+    ``field_from_other_films`` of a single film) gives a zero row; ``total_field`` interpolates the host array of
+    ``FilmSolution.total_field``.  Located once for all entries, as ``interp_current_density_batch``."""
+    valid = ("total_field", "applied_field", "self_field", "field_from_other_films")
+    if dataset not in valid:
+        raise ValueError(f"Unexpected dataset: {dataset}.")
+    solutions, positions = _stage_interp_batch(solutions, positions, film, method)
+    m = len(positions)
+    if not solutions:
+        out = np.zeros((0, m))
+        return _u.Quantity(out, units) if with_units and units is not None else out
+    field_units = solutions[0].field_units
+    convert = units is not None and units != field_units
+    rows = [getattr(s.film_solutions[film], dataset) for s in solutions]
+    out = np.zeros((len(solutions), m))
+    if m and any(r is not None for r in rows):
+        mesh = solutions[0].device.meshes[film]
+        scale = _field_factor(field_units, units) if convert else 1.0
+        out = _interp_batch_device(mesh, rows, 1, positions, None, scale)[:, :, 0]
+    if with_units:
+        return _u.Quantity(out, units if convert else field_units)
+    return out
+
+
 _FIELD_FACTORS: Dict[tuple, float] = {}
 
 
