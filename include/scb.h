@@ -234,9 +234,11 @@ int scb_system_assemble(int64_t n, const double* sites, const double* weights, c
                         const double* sym_scale, scb_stream_t stream);
 
 /* Matrix-free action of the FULL (n x n) operator A on nrhs vectors, sources restricted
- * to `src_idx` (NULL = all vertices):
+ * to `src_idx` (NULL = all vertices; n_src = 0 with a non-NULL src_idx: no source):
  *   out[i,:] (+)= sum_{j in src} A_ij v[j,:],  A_ij = Q_ij w_j - Lambda_j lap_ij - T_ij
  * with Q_ij w_j = -q_ij w_j (i != j), Q_ii w_i = qdw_i.  v, out are [n, nrhs] row-major.
+ * Only the dense part -q_ij w_j reads src_idx; the diagonal and sparse parts act on all of v, so the
+ * sum is over src when v vanishes outside src (as every caller's v does).
  * Replaces the hole slabs `_build_system_1d` @ g[hole] (solve_film.py:285-293,498-503),
  * `Q @ (weights * g)` (solve_film.py:565, with Lambda == NULL: kernel part only) and the
  * check_inversion product (solve_film.py:533-540).  The dense part runs as tiled N-body sums on the
