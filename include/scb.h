@@ -408,6 +408,20 @@ int scb_film_coupling(int64_t m, const double* tgt, double tgt_z, int64_t n, con
                       const double* area, const double* J, int64_t skip_lo, int64_t skip_hi,
                       double prefactor, int64_t nsets, double* out, scb_stream_t stream);
 
+/* scb_film_coupling with every film moved rigidly, per set: set r moves film f by shift[r][f] =
+ * (dx, dy, dz), shift [nsets, nfilms, 3].  The targets belong to film `dst` (0 <= dst < nfilms);
+ * src_film [n] (int32, device) is the film of every packed source row, < 0 for padding rows, which
+ * never move.  Set r equals, bit for bit, an nsets = 1 scb_film_coupling call on the moved inputs
+ *   tgt' = (x_i + shift[r][dst].x, y_i + shift[r][dst].y),  tgt_z' = tgt_z + shift[r][dst].z,
+ *   src'_j = src_j + shift[r][src_film[j]]  (componentwise),  J column r,
+ * because the passes use that call's arithmetic (dx = fl(x_t + o_t) - fl(x_s + o_s), likewise dy and dz;
+ * r^2 = fma(dx, dx, dy dy) + dz^2) and its split of the sources.  Every set has its own geometry, so
+ * nothing is shared between sets: passes of 2 / 1 sets. */
+int scb_film_coupling_translated(int64_t m, const double* tgt, double tgt_z, int64_t n, const double* src,
+                                 const double* area, const double* J, int64_t skip_lo, int64_t skip_hi,
+                                 double prefactor, int64_t nsets, int64_t dst, const int32_t* src_film,
+                                 int64_t nfilms, const double* shift, double* out, scb_stream_t stream);
+
 /* Field of a film's own sheet current at its vertices for `nsets` current-density sets
  * (solve_film.py:415-437 _biot_savart_within_film; the self field of a film with transport terminals):
  *   out[i, s] = prefactor * sum_j area_j (Jx[j,s] (y_i - y_j) - Jy[j,s] (x_i - x_j)) r_ij^-3,

@@ -26,7 +26,7 @@ def _nvcc() -> str:
 
 
 STAMP = LIB + ".stamp"
-ABI_VERSION = 204  # must equal scb_version() of the sources (csrc/api.cu)
+ABI_VERSION = 205  # must equal scb_version() of the sources (csrc/api.cu)
 
 
 def source_digest() -> str:

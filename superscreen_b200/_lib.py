@@ -66,6 +66,9 @@ EXPORTS = {
     "scb_biot_savart": (c_int, [c_int, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_double, c_double, c_int64, c_void_p, c_void_p]),
     "scb_film_coupling": (c_int, [c_int64, c_void_p, c_double, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_int64,
                                   c_double, c_int64, c_void_p, c_void_p]),
+    "scb_film_coupling_translated": (c_int, [c_int64, c_void_p, c_double, c_int64, c_void_p, c_void_p, c_void_p, c_int64,
+                                             c_int64, c_double, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_void_p,
+                                             c_void_p]),
     "scb_biot_savart_within_film": (c_int, [c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_double, c_int64,
                                             c_void_p, c_void_p]),
     "scb_diag_issue_rate": (c_int, [c_int, c_int64, c_void_p, POINTER(c_double), c_void_p]),

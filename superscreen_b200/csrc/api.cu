@@ -18,6 +18,6 @@ void set_error(const char* fmt, ...) {
 void count_launch(int n) { g_launches.fetch_add(n, std::memory_order_relaxed); }
 }  // namespace scb
 
-extern "C" int scb_version(void) { return 204; }
+extern "C" int scb_version(void) { return 205; }
 extern "C" const char* scb_last_error(void) { return scb::g_error; }
 extern "C" int64_t scb_launch_count(void) { return scb::g_launches.load(); }

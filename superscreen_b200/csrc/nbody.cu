@@ -30,6 +30,7 @@ enum : int {
   NB_BOUNDARY = SCB_BS_BOUNDARY,
   NB_KERNEL = 16,    // sum_{j != i} q_ij * payload_j[r], r < NR   (in-plane, 1/r^3)
   NB_COUPLING = 17,  // film-to-film over the packed sources of all films (scb_film_coupling)
+  NB_COUPLING_T = 18,  // NB_COUPLING with a per-set shift of every film (scb_film_coupling_translated)
 };
 
 constexpr int kTile = 256;
@@ -57,17 +58,28 @@ struct NbodyParams {
   double* partial;        // [gridDim.y][m][NACC] partial sums when gridDim.y > 1
 };
 
+// NB_COUPLING_T: set r moves the sources of film f by shift[r][f] and the targets by shift[r][dst].
+// A second kernel argument, so that NbodyParams (and the code of the other kinds) stays as it is.
+struct ShiftTable {
+  const int32_t* src_film;  // [n] film of every packed source row (< 0: padding, never moved)
+  const double* shift;      // [nsets][nfilms][3]
+  int64_t nfilms, dst;
+};
+
 template <int KIND, int NR>
 struct Traits {
   static constexpr int tdim = (KIND == NB_Z || KIND == NB_VECTOR || KIND == NB_VECPOT) ? 3 : 2;
-  // NR = right-hand sides (NB_KERNEL), current-density sets sharing the geometry (film-to-film, NB_Z) or
-  // boundary stream sets sharing the edges (NB_BOUNDARY)
-  static constexpr bool multi = KIND == NB_KERNEL || KIND == NB_FILM_TO_FILM || KIND == NB_COUPLING ||
+  static constexpr bool coupling = KIND == NB_COUPLING || KIND == NB_COUPLING_T;
+  // NR = right-hand sides (NB_KERNEL), current-density sets sharing the geometry (film-to-film, NB_Z),
+  // boundary stream sets sharing the edges (NB_BOUNDARY) or sets with a geometry each (NB_COUPLING_T)
+  static constexpr bool multi = KIND == NB_KERNEL || KIND == NB_FILM_TO_FILM || coupling ||
                                 KIND == NB_BOUNDARY || KIND == NB_Z;
+  // source geometries per tile: NB_COUPLING_T stages the shifted sources of every set, the others share one
+  static constexpr int ngeo = KIND == NB_COUPLING_T ? NR : 1;
   // NB_Z keeps two sums per set (Jx dy, Jy dx) and subtracts them only in nbody_store
   static constexpr int nacc = KIND == NB_Z ? 2 * NR : (multi ? NR : (KIND == NB_VECTOR ? 4 : (KIND == NB_VECPOT ? 2 : 1)));
   static constexpr int npay = KIND == NB_KERNEL ? NR : (multi ? 2 * NR : 2);
-  static constexpr bool has_sz = tdim == 3 || KIND == NB_COUPLING;
+  static constexpr bool has_sz = tdim == 3 || coupling;
 };
 
 // final value(s) of target i from its complete sums
@@ -80,7 +92,7 @@ __device__ __forceinline__ void nbody_store(const NbodyParams& p, int64_t i, con
       double* o = p.out + i * p.ldo + p.rhs0 + r;
       *o = p.accumulate ? *o + pf * acc[r] : pf * acc[r];
     }
-  } else if (KIND == NB_COUPLING || KIND == NB_BOUNDARY) {
+  } else if (Traits<KIND, NR>::coupling || KIND == NB_BOUNDARY) {
 #pragma unroll
     for (int r = 0; r < NR; r++) p.out[i * p.ldo + p.rhs0 + r] = pf * acc[r];
   } else if (KIND == NB_Z) {
@@ -100,12 +112,14 @@ __device__ __forceinline__ void nbody_store(const NbodyParams& p, int64_t i, con
 }
 
 template <int KIND, int NR>
-__global__ void __launch_bounds__(256) nbody_kernel(NbodyParams p) {
+__global__ void __launch_bounds__(256) nbody_kernel(NbodyParams p, ShiftTable st) {
   using T = Traits<KIND, NR>;
   constexpr int TD = T::tdim;
   constexpr int NACC = T::nacc;
   constexpr int NPAY = T::npay;
-  __shared__ double sx[kTile], sy[kTile], sz[T::has_sz ? kTile : 1];
+  constexpr int NG = T::ngeo;
+  constexpr bool SHIFTED = KIND == NB_COUPLING_T;
+  __shared__ double sx[NG * kTile], sy[NG * kTile], sz[T::has_sz ? NG * kTile : 1];
   __shared__ double spay[NPAY][kTile];
 
   const int tid = threadIdx.x;
@@ -119,6 +133,20 @@ __global__ void __launch_bounds__(256) nbody_kernel(NbodyParams p) {
     ty[k] = ok ? p.tgt[TD * ti[k] + 1] : 0.0;
     tz[k] = (ok && TD == 3) ? p.tgt[TD * ti[k] + 2] : 0.0;
   }
+  // NB_COUPLING_T: the targets of every set, moved by the target film's shift once (registers)
+  double gx[TPT][NG], gy[TPT][NG], gz[NG];
+  if (SHIFTED) {
+#pragma unroll
+    for (int g = 0; g < NG; g++) {
+      const double* o = st.shift + ((p.rhs0 + g) * st.nfilms + st.dst) * 3;
+      gz[g] = p.tgt_z + o[2];
+#pragma unroll
+      for (int k = 0; k < TPT; k++) {
+        gx[k][g] = tx[k] + o[0];
+        gy[k][g] = ty[k] + o[1];
+      }
+    }
+  }
   double acc[TPT][NACC];
 #pragma unroll
   for (int k = 0; k < TPT; k++)
@@ -126,17 +154,33 @@ __global__ void __launch_bounds__(256) nbody_kernel(NbodyParams p) {
     for (int a = 0; a < NACC; a++) acc[k][a] = 0.0;
 
   // this CTA's slice of the (virtual, skip range removed) source index space
-  const int64_t n_eff = p.n - (KIND == NB_COUPLING ? p.skip_len : 0);
+  const int64_t n_eff = p.n - (T::coupling ? p.skip_len : 0);
   const int64_t lo = blockIdx.y * p.chunk;
   const int64_t hi = (lo + p.chunk) < n_eff ? (lo + p.chunk) : n_eff;
   for (int64_t base = lo; base < hi; base += kTile) {
     const int64_t v = base + tid;
     __syncthreads();
     if (v < hi) {
-      const int64_t j = (KIND == NB_COUPLING && v >= p.skip_lo) ? v + p.skip_len : v;
+      const int64_t j = (T::coupling && v >= p.skip_lo) ? v + p.skip_len : v;
       const int64_t js = p.src_idx ? p.src_idx[j] : j;
       const double w = p.area[js];
-      if (KIND == NB_COUPLING) {
+      if (SHIFTED) {
+        // every set's shifted source and dz^2, staged once per tile (the arithmetic of a one-set call on
+        // shifted inputs: (x + o) rounded, then the differences)
+        const int f = st.src_film[js];
+        const double x = p.src[3 * js], y = p.src[3 * js + 1], z = p.src[3 * js + 2];
+        const double* Jj = p.J + js * p.ldv + 2 * p.rhs0;
+#pragma unroll
+        for (int g = 0; g < NG; g++) {
+          const double* o = st.shift + ((p.rhs0 + g) * st.nfilms + (f < 0 ? 0 : f)) * 3;
+          sx[g * kTile + tid] = f < 0 ? x : x + o[0];
+          sy[g * kTile + tid] = f < 0 ? y : y + o[1];
+          const double dz = gz[g] - (f < 0 ? z : z + o[2]);
+          sz[g * kTile + tid] = dz * dz;
+          spay[2 * g][tid] = w * Jj[2 * g];
+          spay[2 * g + 1][tid] = w * Jj[2 * g + 1];
+        }
+      } else if (KIND == NB_COUPLING) {
         sx[tid] = p.src[p.sld * js];
         sy[tid] = p.src[p.sld * js + 1];
         const double dz = p.tgt_z - (p.sld == 3 ? p.src[3 * js + 2] : p.tgt_z);
@@ -177,53 +221,60 @@ __global__ void __launch_bounds__(256) nbody_kernel(NbodyParams p) {
     const int cnt = (int)((hi - base) < kTile ? (hi - base) : kTile);
 #pragma unroll 2
     for (int jj = 0; jj < cnt; jj++) {
-      const double xs = sx[jj], ys = sy[jj];
-      const double zs = T::has_sz ? sz[jj] : 0.0;
+      const double xs0 = sx[jj], ys0 = sy[jj];
+      const double zs0 = T::has_sz ? sz[jj] : 0.0;
       double pay[NPAY];
 #pragma unroll
       for (int q = 0; q < NPAY; q++) pay[q] = spay[q][jj];
+      // NG geometries, each shared by NR / NG sets (NG = 1: one r^-3 per pair for all sets)
 #pragma unroll
-      for (int k = 0; k < TPT; k++) {
-        const double dx = tx[k] - xs, dy = ty[k] - ys;
-        double r2 = fma(dx, dx, dy * dy);
-        double dzv = 0.0;
-        if (TD == 3) {
-          dzv = tz[k] - zs;
-          r2 = fma(dzv, dzv, r2);
-        } else if (KIND == NB_COUPLING) {
-          r2 += zs;
-        } else if (KIND == NB_FILM_TO_FILM) {
-          r2 += p.dz2;
-        }
-        if (KIND == NB_VECPOT) {
-          const double inv = inv_r1(r2);
-          acc[k][0] = fma(pay[0], inv, acc[k][0]);
-          acc[k][1] = fma(pay[1], inv, acc[k][1]);
-        } else {
-          double k3 = inv_r3(r2);
-          if (KIND == NB_KERNEL) {
-            k3 = r2 > 0.0 ? k3 : 0.0;  // q_ii = 0 (distance.py:104-105)
+      for (int g = 0; g < NG; g++) {
+        const double xs = g == 0 ? xs0 : sx[g * kTile + jj], ys = g == 0 ? ys0 : sy[g * kTile + jj];
+        const double zs = g == 0 ? zs0 : sz[g * kTile + jj];
 #pragma unroll
-            for (int r = 0; r < NR; r++) acc[k][r] = fma(pay[r], k3, acc[k][r]);
-          } else if (KIND == NB_FILM_TO_FILM || KIND == NB_COUPLING) {
-            const double kdy = k3 * dy, kdx = k3 * dx;
+        for (int k = 0; k < TPT; k++) {
+          const double dx = (SHIFTED ? gx[k][g] : tx[k]) - xs, dy = (SHIFTED ? gy[k][g] : ty[k]) - ys;
+          double r2 = fma(dx, dx, dy * dy);
+          double dzv = 0.0;
+          if (TD == 3) {
+            dzv = tz[k] - zs;
+            r2 = fma(dzv, dzv, r2);
+          } else if (T::coupling) {
+            r2 += zs;
+          } else if (KIND == NB_FILM_TO_FILM) {
+            r2 += p.dz2;
+          }
+          if (KIND == NB_VECPOT) {
+            const double inv = inv_r1(r2);
+            acc[k][0] = fma(pay[0], inv, acc[k][0]);
+            acc[k][1] = fma(pay[1], inv, acc[k][1]);
+          } else {
+            double k3 = inv_r3(r2);
+            if (KIND == NB_KERNEL) {
+              k3 = r2 > 0.0 ? k3 : 0.0;  // q_ii = 0 (distance.py:104-105)
 #pragma unroll
-            for (int r = 0; r < NR; r++) acc[k][r] = fma(pay[2 * r], kdy, fma(-pay[2 * r + 1], kdx, acc[k][r]));
-          } else if (KIND == NB_BOUNDARY) {
+              for (int r = 0; r < NR; r++) acc[k][r] = fma(pay[r], k3, acc[k][r]);
+            } else if (KIND == NB_FILM_TO_FILM || T::coupling) {
+              const double kdy = k3 * dy, kdx = k3 * dx;
 #pragma unroll
-            for (int r = 0; r < NR; r++) acc[k][r] = fma(-k3, fma(pay[2 * r], dx, pay[2 * r + 1] * dy), acc[k][r]);
-          } else if (KIND == NB_Z) {
+              for (int r = g * (NR / NG); r < (g + 1) * (NR / NG); r++)
+                acc[k][r] = fma(pay[2 * r], kdy, fma(-pay[2 * r + 1], kdx, acc[k][r]));
+            } else if (KIND == NB_BOUNDARY) {
 #pragma unroll
-            for (int r = 0; r < NR; r++) {
-              acc[k][2 * r] = fma(k3 * pay[2 * r], dy, acc[k][2 * r]);              // Jx_dy
-              acc[k][2 * r + 1] = fma(k3 * pay[2 * r + 1], dx, acc[k][2 * r + 1]);  // Jy_dx
+              for (int r = 0; r < NR; r++) acc[k][r] = fma(-k3, fma(pay[2 * r], dx, pay[2 * r + 1] * dy), acc[k][r]);
+            } else if (KIND == NB_Z) {
+#pragma unroll
+              for (int r = 0; r < NR; r++) {
+                acc[k][2 * r] = fma(k3 * pay[2 * r], dy, acc[k][2 * r]);              // Jx_dy
+                acc[k][2 * r + 1] = fma(k3 * pay[2 * r + 1], dx, acc[k][2 * r + 1]);  // Jy_dx
+              }
+            } else {                                        // NB_VECTOR
+              const double px = k3 * pay[0], py = k3 * pay[1];
+              acc[k][0] = fma(px, dy, acc[k][0]);   // Jx_dy
+              acc[k][1] = fma(py, dx, acc[k][1]);   // Jy_dx
+              acc[k][2] = fma(px, dzv, acc[k][2]);  // Jx_dz
+              acc[k][3] = fma(py, dzv, acc[k][3]);  // Jy_dz
             }
-          } else {                                        // NB_VECTOR
-            const double px = k3 * pay[0], py = k3 * pay[1];
-            acc[k][0] = fma(px, dy, acc[k][0]);   // Jx_dy
-            acc[k][1] = fma(py, dx, acc[k][1]);   // Jy_dx
-            acc[k][2] = fma(px, dzv, acc[k][2]);  // Jx_dz
-            acc[k][3] = fma(py, dzv, acc[k][3]);  // Jy_dz
           }
         }
       }
@@ -274,21 +325,23 @@ __global__ void __launch_bounds__(128) nbody_reduce_kernel(NbodyParams p, int ns
 static bool g_pool_set[64] = {};
 
 template <int KIND, int NR>
-static int launch_nbody(NbodyParams p, cudaStream_t s) {
+static int launch_nbody(NbodyParams p, cudaStream_t s, ShiftTable st = {}) {
   if (p.m == 0) return SCB_OK;
   constexpr int NACC = Traits<KIND, NR>::nacc;
-  const int64_t n_eff = p.n - (KIND == NB_COUPLING ? p.skip_len : 0);
+  const int64_t n_eff = p.n - (Traits<KIND, NR>::coupling ? p.skip_len : 0);
   const int64_t ctas_x = ceil_div(p.m, 256 * TPT);
   // One balanced wave: every CTA does the same amount of work, so the source range is split until the
   // grid just fills the resident-CTA capacity of the device (a CTA keeps at least one source tile).
   // NB_Z passes of several sets split as the single-set pass does, whatever their own occupancy: the
   // split fixes the summation order, so every set of a multi-set call has the bits of a one-set call.
-  constexpr int CAP_NR = KIND == NB_Z ? 1 : NR;
+  // NB_COUPLING_T passes split as the one-set NB_COUPLING pass does, for the same reason.
+  constexpr int CAP_NR = (KIND == NB_Z || KIND == NB_COUPLING_T) ? 1 : NR;
+  constexpr int CAP_KIND = KIND == NB_COUPLING_T ? NB_COUPLING : KIND;
   static int capacity = 0;  // per instantiation; all devices of a node are identical
   if (capacity == 0) {
     int per_sm = 0, sms = 0, dev = 0;
     SCB_CUDA(cudaGetDevice(&dev));
-    SCB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, nbody_kernel<KIND, CAP_NR>, 256, 0));
+    SCB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, nbody_kernel<CAP_KIND, CAP_NR>, 256, 0));
     SCB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     capacity = per_sm * sms > 0 ? per_sm * sms : 148;
   }
@@ -311,7 +364,7 @@ static int launch_nbody(NbodyParams p, cudaStream_t s) {
     }
     SCB_CUDA(cudaMallocAsync(&p.partial, sizeof(double) * (size_t)(split * p.m * NACC), s));
   }
-  nbody_kernel<KIND, NR><<<dim3((unsigned)ctas_x, (unsigned)split), 256, 0, s>>>(p);
+  nbody_kernel<KIND, NR><<<dim3((unsigned)ctas_x, (unsigned)split), 256, 0, s>>>(p, st);
   SCB_LAUNCH_CHECK();
   if (split > 1) {
     nbody_reduce_kernel<KIND, NR><<<(unsigned)ceil_div(p.m, 128 / NACC), 128, 0, s>>>(p, (int)split);
@@ -687,6 +740,37 @@ extern "C" int scb_film_coupling(int64_t m, const double* tgt, double tgt_z, int
     else if (nsets - k >= 4) { rc = launch_nbody<NB_COUPLING, 4>(p, s); k += 4; }
     else if (nsets - k >= 2) { rc = launch_nbody<NB_COUPLING, 2>(p, s); k += 2; }
     else { rc = launch_nbody<NB_COUPLING, 1>(p, s); k += 1; }
+    if (rc) return rc;
+  }
+  return SCB_OK;
+}
+
+extern "C" int scb_film_coupling_translated(int64_t m, const double* tgt, double tgt_z, int64_t n, const double* src,
+                                            const double* area, const double* J, int64_t skip_lo, int64_t skip_hi,
+                                            double prefactor, int64_t nsets, int64_t dst, const int32_t* src_film,
+                                            int64_t nfilms, const double* shift, double* out, scb_stream_t stream) {
+  SCB_CHECK_ARG(m >= 0 && n >= 0 && nsets >= 1, "bad sizes");
+  SCB_CHECK_ARG(0 <= skip_lo && skip_lo <= skip_hi && skip_hi <= n, "skip range must lie inside [0, n]");
+  SCB_CHECK_ARG(nfilms >= 1 && 0 <= dst && dst < nfilms, "dst must lie in [0, nfilms)");
+  cudaStream_t s = (cudaStream_t)stream;
+  if (m == 0) return SCB_OK;
+  if (skip_lo == 0 && skip_hi == n) {  // no other film: the field vanishes
+    SCB_CUDA(cudaMemsetAsync(out, 0, sizeof(double) * (size_t)(m * nsets), s));
+    return SCB_OK;
+  }
+  NbodyParams p{};
+  p.m = m; p.tgt = tgt; p.tgt_z = tgt_z; p.n = n; p.src = src; p.area = area; p.J = J; p.ldv = 2 * nsets;
+  p.skip_lo = skip_lo; p.skip_len = skip_hi - skip_lo; p.prefactor = prefactor; p.out = out; p.ldo = nsets;
+  p.sld = 3;
+  const ShiftTable st{src_film, shift, nfilms, dst};
+  // No r^-3 to share between sets: a pass of several sets only saves target loads and launches.  Passes
+  // of 2 (80 registers, 20 KB of shared memory: 3 CTAs per SM); a 4-set pass needs 136 registers, one CTA.
+  int64_t k = 0;
+  while (k < nsets) {
+    p.rhs0 = k;
+    int rc;
+    if (nsets - k >= 2) { rc = launch_nbody<NB_COUPLING_T, 2>(p, s, st); k += 2; }
+    else { rc = launch_nbody<NB_COUPLING_T, 1>(p, s, st); k += 1; }
     if (rc) return rc;
   }
   return SCB_OK;

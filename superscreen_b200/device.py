@@ -283,6 +283,16 @@ class CompositePolygon(Polygon):
     def _mapped(self, points, inplace):
         raise NotImplementedError("Affine maps of composite polygons are not supported; transform the parts.")
 
+    def translate(self, dx: float = 0.0, dy: float = 0.0, inplace: bool = False) -> "CompositePolygon":
+        """Every ring moved by ``(dx, dy)``, as ``Polygon.translate`` moves its points (so that
+        ``Device.translate`` and the translated entries of ``solve_batch`` can move a composite film or hole)."""
+        shift = np.array([dx, dy], dtype=float)
+        polygon = self if inplace else self.copy()
+        polygon._add = [close_curve(orient_ccw(r + shift)) for r in self._add]
+        polygon._sub = [close_curve(orient_ccw(r + shift)) for r in self._sub]
+        polygon._points = np.concatenate(polygon._add, axis=0)
+        return polygon
+
     def contains_points(self, points, index: bool = False, radius: float = 0):
         pts = np.atleast_2d(points)
         mask = np.zeros(len(pts), dtype=bool)

@@ -334,9 +334,16 @@ class Solution:
     def __init__(self, *, device: Device, film_solutions: Dict[str, FilmSolution], applied_field_func: Callable,
                  field_units: str, current_units: str, circulating_currents: Optional[Dict[str, float]] = None,
                  terminal_currents: Optional[Dict[str, float]] = None, vortices=None,
-                 solver: str = "superscreen_b200.solve", _device_is_copy: bool = False):
-        # (the solver hands one private copy of the device to all the solutions of a call)
-        self.device = device if _device_is_copy else device.copy(with_mesh=True, copy_mesh=False)
+                 solver: str = "superscreen_b200.solve", _device_is_copy: bool = False,
+                 _device_builder: Optional[Callable[[], Device]] = None):
+        # (the solver hands one private copy of the device to all the solutions of a call; a translated
+        # entry of solve_batch gets a builder instead, shared by the entries with the same translation, that
+        # makes the translated device on first access)
+        self._device_builder = _device_builder
+        if _device_builder is None:
+            self.device = device if _device_is_copy else device.copy(with_mesh=True, copy_mesh=False)
+        else:
+            self._device = None
         self.film_solutions = film_solutions
         self.applied_field_func = applied_field_func
         self.circulating_currents = circulating_currents or {}
@@ -346,6 +353,16 @@ class Solution:
         self._current_units = current_units
         self._solver = solver
         self._time_created = dt.datetime.now()
+
+    @property
+    def device(self) -> Device:
+        if self._device is None:
+            self._device = self._device_builder()
+        return self._device
+
+    @device.setter
+    def device(self, device: Device) -> None:
+        self._device = device
 
     @property
     def version_info(self) -> Dict[str, str]:

@@ -10,15 +10,17 @@ from __future__ import annotations
 import copy
 import itertools
 import logging
+import numbers
 import os
 from dataclasses import dataclass, field
-from typing import Callable, Dict, List, Optional, Sequence, Union
+from typing import Callable, Dict, List, Optional, Sequence, Tuple, Union
 
 import numpy as np
 
 from .. import _lib
 from .. import units as _u
 from ..device import Device
+from ..mesh import Mesh
 from ..solution import FilmSolution, Solution, Vortex
 from ..sources import ConstantField
 from .solve_film import (  # noqa: F401  (TerminalSystems, solve_film: names the reference module exposes)
@@ -204,10 +206,13 @@ def _to_host(t) -> np.ndarray:
     return stage.numpy()
 
 
-def _solutions_from_host(device, host, film_names, host_fields, field_conversion, kwargs_list, batched):
+def _solutions_from_host(device, host, film_names, host_fields, field_conversion, kwargs_list, batched,
+                         device_builders=None):
     """HostResults (parallel.ResultPacker) -> [[Solution per batch entry] per stored iterate]
     (reference solve_film.py:566-573: fields are handed out in ``field_units``).  The arrays of the
-    FilmSolutions are views of the one downloaded buffer; the applied field never left the host."""
+    FilmSolutions are views of the one downloaded buffer; the applied field never left the host.
+    ``device_builders`` (batched only): per entry ``None`` (the shared copy of ``device``) or the builder of
+    its translated device."""
     applied = {name: host_fields[name] / field_conversion for name in film_names}
     shared = device.copy(with_mesh=True, copy_mesh=False)  # one copy shared by the solutions of this call
     out = []
@@ -220,20 +225,28 @@ def _solutions_from_host(device, host, film_names, host_fields, field_conversion
                 film_solutions[name] = FilmSolution(
                     stream=g, current_density=J, applied_field=applied[name][b] if batched else applied[name],
                     self_field=self_field, field_from_other_films=other)
-            row.append(Solution(device=shared, film_solutions=film_solutions, _device_is_copy=True, **kwargs))
+            row.append(Solution(device=shared, film_solutions=film_solutions, _device_is_copy=True,
+                                _device_builder=None if device_builders is None else device_builders[b], **kwargs))
         out.append(row)
     return out
 
 
-def _evaluate_applied_field(applied_field, device, film_info, meshes, field_conversion, films=None):
-    """reference solver/solve.py:422-436 -> {film: host float64 (n,) in solver units}"""
+def _evaluate_applied_field(applied_field, device, film_info, meshes, field_conversion, films=None, moves=None):
+    """reference solver/solve.py:422-436 -> {film: host float64 (n,) in solver units}.  ``moves``
+    ({layer: (dx, dy, dz)}): the field at the vertices of those layers' films moved as ``Device.translate``
+    moves them (``sites + (dx, dy)``, ``z0 + dz``)."""
     out = {}
     for film, mesh in meshes.items():
         if films is not None and film not in films:
             continue
         layer = device.layers[film_info[film].layer]
-        z0 = layer.z0 * np.ones(len(mesh.sites))
-        Hz_applied = np.squeeze(applied_field(mesh.sites[:, 0], mesh.sites[:, 1], z0) * field_conversion)
+        sites, z0 = mesh.sites, layer.z0
+        if moves and film_info[film].layer in moves:
+            dx, dy, dz = moves[film_info[film].layer]
+            sites = np.asarray(sites) + np.array([[dx, dy]], dtype=float) if (dx or dy) else sites
+            z0 = z0 + dz
+        z0 = z0 * np.ones(len(sites))
+        Hz_applied = np.squeeze(applied_field(sites[:, 0], sites[:, 1], z0) * field_conversion)
         Hz_applied = np.asarray(Hz_applied, dtype=np.float64)
         if Hz_applied.ndim != 1:
             raise ValueError(
@@ -245,9 +258,9 @@ def _evaluate_applied_field(applied_field, device, film_info, meshes, field_conv
 
 
 def _packed_sources(model: "FactorizedModel", layout, z0s, dev):
-    """Static part of the film-to-film coupling: vertices (x, y, z0) and vertex areas of ALL films in
-    the packed layout of ``parallel.FilmLayout`` (padding rows: far away, zero area).  Built once per
-    model and device."""
+    """Static part of the film-to-film coupling: vertices (x, y, z0), vertex areas and the film index
+    (position in ``layout.films``, int32) of ALL films in the packed layout of ``parallel.FilmLayout``
+    (padding rows: far away, zero area, film -1).  Built once per model and device."""
     torch = _torch()
     cache = model.__dict__.setdefault("_packed_cache", {})
     key = (str(dev), tuple(layout.films), layout.world)
@@ -255,24 +268,28 @@ def _packed_sources(model: "FactorizedModel", layout, z0s, dev):
     if hit is None:
         src = torch.full((layout.total, 3), 1e30, dtype=torch.float64, device=dev)
         area = torch.zeros(layout.total, dtype=torch.float64, device=dev)
-        for name in layout.films:
+        film = torch.full((layout.total,), -1, dtype=torch.int32, device=dev)
+        for k, name in enumerate(layout.films):
             d = model.device.meshes[name]._data
             lo, hi = layout.rows(name)
             src[lo:hi, :2] = d.sites.to(dev)
             src[lo:hi, 2] = z0s[name]
             area[lo:hi] = d.t["vertex_areas"].to(dev)
-        hit = cache[key] = (src, area)
+            film[lo:hi] = k
+        hit = cache[key] = (src, area, film)
     return hit
 
 
 def _run(model: "FactorizedModel", applied_fields, circ_by_film, vortex_flux, iterations, check_inversion,
          field_conversion: float, batch: Optional[int] = None, last_only: bool = False, gather: bool = True,
          terminal_currents: Optional[List[Dict[str, Dict[str, float]]]] = None,
-         vortices: Optional[List[Dict[str, List[Vortex]]]] = None):
+         vortices: Optional[List[Dict[str, List[Vortex]]]] = None, shifts: Optional[np.ndarray] = None):
     """Runs the solve + film-to-film iterations on the device for single or batched right-hand
     sides.  ``terminal_currents`` (batched only): one ``{film: {terminal: current}}`` dict per entry
     (default: the model's for every entry).  ``vortices`` (batched only): one ``{film: [Vortex]}`` dict per
-    entry (default: the model's vortices for every entry).  Everything stays on the device until the
+    entry (default: the model's vortices for every entry).  ``shifts`` (batched only): ``(B, films, 3)``, the
+    rigid shift of every film per entry, films in device order; the film-to-film coupling then runs on the moved
+    geometry (``scb_film_coupling_translated``).  Everything stays on the device until the
     end: every owned film's result of every stored iterate is packed into one buffer (``parallel.ResultPacker``), replicated over the ranks by one
     all-gather if ``gather`` and downloaded once.  Returns ``parallel.HostResults``."""
     torch = _torch()
@@ -337,6 +354,9 @@ def _run(model: "FactorizedModel", applied_fields, circ_by_film, vortex_flux, it
             want_self_field=it in iterates)  # (the self field of an iterate that is not stored is never used)
 
     inv4pi = 1.0 / (4.0 * np.pi)
+    shift_table = None
+    if shifts is not None and multi:
+        shift_table = _upload(np.ascontiguousarray(shifts, dtype=np.float64), dev)
 
     def coupling_fn(dst, J_all):
         with _lib.nvtx_range(f"scb.film_coupling[{dst}]"):
@@ -344,14 +364,20 @@ def _run(model: "FactorizedModel", applied_fields, circ_by_film, vortex_flux, it
 
     def _coupling_fn(dst, J_all):
         # sum over every other film of biot_savart_film_to_film (reference solve.py:495-515): one launch
-        src, area = _packed_sources(model, layout, z0s, dev)
+        src, area, src_film = _packed_sources(model, layout, z0s, dev)
         d = meshes[dst]._data
         lo, hi = layout.rows(dst)
         with torch.cuda.device(dev):
             out = torch.empty((d.n, batch) if batch is not None else (d.n,), dtype=torch.float64, device=dev)
-            _lib.check(L.scb_film_coupling(d.n, _lib.ptr(d.sites), z0s[dst], layout.total, _lib.ptr(src),
-                                           _lib.ptr(area), _lib.ptr(J_all), lo, hi, inv4pi,
-                                           batch if batch is not None else 1, _lib.ptr(out), _lib.stream_ptr()))
+            if shift_table is None:
+                _lib.check(L.scb_film_coupling(d.n, _lib.ptr(d.sites), z0s[dst], layout.total, _lib.ptr(src),
+                                               _lib.ptr(area), _lib.ptr(J_all), lo, hi, inv4pi,
+                                               batch if batch is not None else 1, _lib.ptr(out), _lib.stream_ptr()))
+            else:
+                _lib.check(L.scb_film_coupling_translated(
+                    d.n, _lib.ptr(d.sites), z0s[dst], layout.total, _lib.ptr(src), _lib.ptr(area), _lib.ptr(J_all),
+                    lo, hi, inv4pi, batch, layout.films.index(dst), _lib.ptr(src_film), len(layout.films),
+                    _lib.ptr(shift_table), _lib.ptr(out), _lib.stream_ptr()))
         return out
 
     # the films of one Jacobi step are independent and each is latency-bound (getrs sweeps, small
@@ -508,10 +534,95 @@ def _batch_vortices(device: Device, vortices, B: int) -> List[Dict[str, List[Vor
     return out
 
 
+def _batch_translations(device: Device, translations, B: int,
+                        vortices: Sequence[Sequence[Vortex]]) -> Optional[List[Dict[str, Tuple[float, float, float]]]]:
+    """Validates the per-entry layer translations of ``solve_batch`` before any device work, naming the
+    offending entry.  ``vortices``: the vortices of every entry.  Returns one ``{layer: (dx, dy, dz)}`` dict per
+    entry holding the layers it moves (a zero shift moves nothing), or ``None`` when no entry moves anything."""
+    if len(translations) != B:
+        raise ValueError(f"applied_fields and translations must have the same length "
+                         f"(got {B} and {len(translations)}).")
+    out = []
+    for b, entry in enumerate(translations):
+        entry = {} if entry is None else entry
+        if not isinstance(entry, dict):
+            raise TypeError(f"translations[{b}]: expected None or a dict {{layer: (dx, dy) | (dx, dy, dz)}}, "
+                            f"but got {entry!r}.")
+        moves = {}
+        for layer, value in entry.items():
+            if layer not in device.layers:
+                raise KeyError(f"translations[{b}]: the device has no layer {layer!r}.")
+            shift = tuple(value) if isinstance(value, (tuple, list, np.ndarray)) else ()
+            if not (len(shift) in (2, 3) and all(isinstance(v, numbers.Real) and np.isfinite(v) for v in shift)):
+                raise ValueError(f"translations[{b}]: the shift of layer {layer!r} must be 2 or 3 finite reals "
+                                 f"(dx, dy[, dz]), but got {value!r}.")
+            shift = tuple(float(v) for v in shift) + (0.0,) * (3 - len(shift))
+            if any(shift):
+                moves[layer] = shift
+        for layer in moves:
+            if callable(device.layers[layer].Lambda):
+                raise ValueError(f"translations[{b}]: layer {layer!r} has a position-dependent Lambda, so moving it "
+                                 "would change its factorization.")
+        for vortex in vortices[b]:
+            layer = device.films[vortex.film].layer
+            if layer in moves:
+                raise ValueError(f"translations[{b}]: {vortex!r} is in layer {layer!r}, which the entry moves; "
+                                 "vortices in moved layers are not supported.")
+        out.append(moves)
+    return out if any(out) else None
+
+
+def _translated_device(device: Device, moves: Dict[str, Tuple[float, float, float]]) -> Device:
+    """A copy of ``device`` with the layers in ``moves`` (``{layer: (dx, dy, dz)}``) moved as
+    ``Device.translate`` moves a whole device: every polygon of those layers (films, holes, terminals,
+    abstract regions) by ``(dx, dy)``, the meshes of their films rebuilt from ``sites + (dx, dy)``, ``z0`` by
+    ``dz``.  The meshes of the other films are shared with ``device``."""
+    out = device.copy(with_mesh=False)
+    for polygon in out.get_polygons():
+        if polygon.layer in moves:
+            polygon.translate(*moves[polygon.layer][:2], inplace=True)
+    meshes = dict(device.meshes)
+    for name, film in device.films.items():
+        dx, dy, _ = moves.get(film.layer, (0.0, 0.0, 0.0))
+        if dx or dy:
+            mesh = device.meshes[name]
+            meshes[name] = Mesh.from_triangulation(np.asarray(mesh.sites) + np.array([[dx, dy]], dtype=float),
+                                                   np.asarray(mesh.elements))
+    out.meshes = meshes
+    for layer, (_, _, dz) in moves.items():
+        if dz:
+            out.layers[layer].z0 += dz
+    return out
+
+
+def _device_builders(device: Device, moves: List[Dict[str, Tuple[float, float, float]]]):
+    """Per entry ``None`` (nothing moves) or a function that builds the entry's translated device on first
+    call; entries with the same translation share the function and so the device."""
+    by_key = {}
+    out = []
+    for entry in moves:
+        if not entry:
+            out.append(None)
+            continue
+        key = tuple(sorted(entry.items()))
+        if key not in by_key:
+            built = []
+
+            def build(entry=entry, built=built):
+                if not built:
+                    built.append(_translated_device(device, entry))
+                return built[0]
+
+            by_key[key] = build
+        out.append(by_key[key])
+    return out
+
+
 def solve_batch(*, model: FactorizedModel, applied_fields: Sequence[Optional[Callable]],
                 circulating_currents: Optional[Sequence[Dict[str, float]]] = None,
                 terminal_currents: Optional[Sequence[Dict[str, Dict[str, Union[float, str]]]]] = None,
                 vortices: Optional[Sequence[Sequence[Vortex]]] = None,
+                translations: Optional[Sequence[Optional[Dict[str, Sequence[float]]]]] = None,
                 field_units: str = "mT",
                 iterations: int = 0, check_inversion: bool = False, last_only: bool = False,
                 gather: bool = True, _solver: str = "superscreen_b200.solve_batch") -> List[List[Solution]]:
@@ -533,7 +644,22 @@ def solve_batch(*, model: FactorizedModel, applied_fields: Sequence[Optional[Cal
     checks them (``TypeError`` for an item that is not a ``Vortex``, ``KeyError`` for an unknown film,
     ``ValueError`` for a vortex outside its film or inside a hole, naming the entry) before any device
     work.  Each vortex enters its own entry's right-hand side as a sparse correction, so a scan over
-    vortex positions costs one batched solve, not one solve per position.  With
+    vortex positions costs one batched solve, not one solve per position.
+
+    ``translations`` has one ``None`` or ``{layer: (dx, dy) | (dx, dy, dz)}`` dict per entry (in
+    ``device.length_units``): every film, hole, terminal and abstract region of a listed layer moves rigidly
+    by ``(dx, dy)`` and the layer by ``dz``; other layers stay put.  ``model_b`` is then the factorization of
+    the device with those layers moved as ``Device.translate`` moves them.  Only the applied field (evaluated
+    at the moved vertices) and the film-to-film coupling depend on where a film sits, so a scan over the
+    positions of a layer stack (a scanning SQUID over a sample) costs one batched solve against one
+    factorization per film.  A layer with a position-dependent Lambda, or that holds a vortex of the entry,
+    cannot move (``ValueError``, naming the entry); so do unknown layers (``KeyError``) and shifts that are
+    not 2 or 3 finite reals (``ValueError``).  Films with terminals may move.  ``Solution.device`` of an
+    entry that moves something is the moved device, built on first access and shared by the entries with
+    the same translation, so ``hole_fluxoid``, ``polygon_fluxoid`` and ``field_at_position`` work on it
+    unchanged (an explicit fluxoid contour must be moved with its layer by the caller).  When no entry moves
+    anything the call is the one without ``translations``.  Multi-rank models replicate the small shift
+    table; that path is untested, as it is for vortices.  With
     ``last_only`` only the final iterate is brought to the host (``out[b]`` has one element).
     With a multi-rank model, ``gather=False`` skips the replication of the results: every rank's
     solutions then hold only the films it owns (enough for per-film post-processing such as the
@@ -559,6 +685,14 @@ def solve_batch(*, model: FactorizedModel, applied_fields: Sequence[Optional[Cal
     if vortices is not None:
         vortices_by_film = _batch_vortices(device, vortices, B)
         vortices = [[] if entry is None else list(entry) for entry in vortices]
+    moves = None
+    if translations is not None:
+        if vortices is not None:
+            entry_vortices = vortices
+        else:
+            entry_vortices = [list(itertools.chain.from_iterable(model.vortices.values()))
+                              if isinstance(model.vortices, dict) else list(model.vortices)] * B
+        moves = _batch_translations(device, translations, B, entry_vortices)
     current_units = model.current_units
     length_units = device.length_units
     field_conversion = field_conversion_factor(field_units, current_units, length_units=length_units).magnitude
@@ -567,15 +701,23 @@ def solve_batch(*, model: FactorizedModel, applied_fields: Sequence[Optional[Cal
     owned = _owned_films(model)
     film_names = [f for f in device.films if gather or f in owned]
     with _lib.nvtx_range("scb.solve_batch.fields"):
-        # (a field function that appears several times in the batch is evaluated once)
+        # (a field function that appears several times in the batch is evaluated once per film and
+        # translation of the film's layer)
         evaluated = {}
         per_b = []
-        for f in funcs:
-            hit = evaluated.get(id(f))
-            if hit is None:
-                hit = evaluated[id(f)] = _evaluate_applied_field(f, device, model.film_info, device.meshes,
-                                                                 field_conversion, films=film_names)
-            per_b.append(hit)
+        for b, f in enumerate(funcs):
+            entry_moves = {} if moves is None else moves[b]
+            fields = {}
+            for name in film_names:
+                layer = model.film_info[name].layer
+                key = (id(f), name, entry_moves.get(layer))
+                hit = evaluated.get(key)
+                if hit is None:
+                    hit = evaluated[key] = _evaluate_applied_field(f, device, model.film_info, device.meshes,
+                                                                   field_conversion, films=[name],
+                                                                   moves=entry_moves)[name]
+                fields[name] = hit
+            per_b.append(fields)
         host_fields = {name: np.stack([h[name] for h in per_b], axis=0) for name in film_names}  # (B, n) per film
         dev_fields = {}
         circ_by_film = {}
@@ -601,9 +743,13 @@ def solve_batch(*, model: FactorizedModel, applied_fields: Sequence[Optional[Cal
             circ_by_film[name] = {hole: tables[dev][k] for k, (film, hole) in enumerate(hole_rows.get(dev, []))
                                   if film == name}
     vortex_flux = _u.PHI_0 / _u.MU_0 * _u.conversion_factor("A * m", f"({current_units}) * ({length_units})")
+    shifts = None
+    if moves is not None:
+        shifts = np.array([[entry.get(film.layer, (0.0, 0.0, 0.0)) for film in device.films.values()]
+                           for entry in moves], dtype=np.float64)  # (B, films, 3)
     host = _run(model, dev_fields, circ_by_film, vortex_flux, iterations, check_inversion, field_conversion,
                 batch=B, last_only=last_only, gather=gather, terminal_currents=terminal_currents,
-                vortices=vortices_by_film)
+                vortices=vortices_by_film, shifts=shifts)
     kwargs_list = [dict(applied_field_func=funcs[b], field_units=field_units, current_units=current_units,
                         circulating_currents=dict(circulating_currents[b]),
                         terminal_currents=model.terminal_currents if terminal_currents is None
@@ -612,7 +758,9 @@ def solve_batch(*, model: FactorizedModel, applied_fields: Sequence[Optional[Cal
                    for b in range(B)]
     with _lib.nvtx_range("scb.solve_batch.solutions"):
         per_iter_solutions = _solutions_from_host(device, host, film_names, host_fields, field_conversion,
-                                                  kwargs_list, batched=True)
+                                                  kwargs_list, batched=True,
+                                                  device_builders=None if moves is None
+                                                  else _device_builders(device, moves))
     return [[it[b] for it in per_iter_solutions] for b in range(B)]
 
 
