@@ -389,9 +389,9 @@ enum scb_bs_kind {
 /* out = prefactor * sum_j area_j * kernel(tgt_i, src_j, J_j).  nsets > 1 evaluates `nsets`
  * current-density sets J[nsets, n, 2] against the same geometry, out[nsets, m(, c)]; for
  * SCB_BS_BOUNDARY the sets are the columns of area[n, nsets] and out[m, nsets] (see above).
- * SCB_BS_FILM_TO_FILM, SCB_BS_Z and SCB_BS_BOUNDARY evaluate r^-3 of a pair once for up to 8 sets
- * (passes of 8 / 4 / 2 / 1 sets); SCB_BS_VECTOR and SCB_BS_VECTOR_POTENTIAL run one pass per set.
- * Every set of an SCB_BS_Z call has the bits of an nsets = 1 call on that set alone: the passes
+ * Every kind evaluates r^-3 (SCB_BS_VECTOR_POTENTIAL: r^-1) of a pair once for up to 8 sets
+ * (passes of 8 / 4 / 2 / 1 sets).  Every set of an SCB_BS_Z, SCB_BS_VECTOR or
+ * SCB_BS_VECTOR_POTENTIAL call has the bits of an nsets = 1 call on that set alone: the passes
  * share its arithmetic and its split of the sources, which depends only on (m, n). */
 int scb_biot_savart(int kind, int64_t m, const double* tgt, int64_t n, const double* src,
                     const double* area, const double* J, double dz, double prefactor,

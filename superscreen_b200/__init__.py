@@ -11,7 +11,7 @@ from .fluxoid import find_fluxoid_solution, make_fluxoid_polygons
 from .mesh import Mesh, MeshOperators
 from .meshgen import generate_mesh
 from .solution import (FilmSolution, Fluxoid, Solution, Vortex, field_at_position_batch, interp_current_density_batch,
-                       interp_field_batch)
+                       interp_field_batch, screening_field_at_position_batch, vector_potential_at_position_batch)
 from .solver import (
     FactorizedModel,
     FilmInfo,

@@ -70,15 +70,15 @@ template <int KIND, int NR>
 struct Traits {
   static constexpr int tdim = (KIND == NB_Z || KIND == NB_VECTOR || KIND == NB_VECPOT) ? 3 : 2;
   static constexpr bool coupling = KIND == NB_COUPLING || KIND == NB_COUPLING_T;
-  // NR = right-hand sides (NB_KERNEL), current-density sets sharing the geometry (film-to-film, NB_Z),
-  // boundary stream sets sharing the edges (NB_BOUNDARY) or sets with a geometry each (NB_COUPLING_T)
-  static constexpr bool multi = KIND == NB_KERNEL || KIND == NB_FILM_TO_FILM || coupling ||
-                                KIND == NB_BOUNDARY || KIND == NB_Z;
+  // NR = right-hand sides (NB_KERNEL), current-density sets sharing the geometry (film-to-film, NB_Z,
+  // NB_VECTOR, NB_VECPOT), boundary stream sets sharing the edges (NB_BOUNDARY) or sets with a geometry each
+  // (NB_COUPLING_T)
   // source geometries per tile: NB_COUPLING_T stages the shifted sources of every set, the others share one
   static constexpr int ngeo = KIND == NB_COUPLING_T ? NR : 1;
-  // NB_Z keeps two sums per set (Jx dy, Jy dx) and subtracts them only in nbody_store
-  static constexpr int nacc = KIND == NB_Z ? 2 * NR : (multi ? NR : (KIND == NB_VECTOR ? 4 : (KIND == NB_VECPOT ? 2 : 1)));
-  static constexpr int npay = KIND == NB_KERNEL ? NR : (multi ? 2 * NR : 2);
+  // NB_Z keeps two sums per set (Jx dy, Jy dx) and subtracts them only in nbody_store, NB_VECTOR four
+  // (Jx dy, Jy dx, Jx dz, Jy dz), NB_VECPOT two (Jx, Jy)
+  static constexpr int nacc = (KIND == NB_Z || KIND == NB_VECPOT) ? 2 * NR : (KIND == NB_VECTOR ? 4 * NR : NR);
+  static constexpr int npay = KIND == NB_KERNEL ? NR : 2 * NR;
   static constexpr bool has_sz = tdim == 3 || coupling;
 };
 
@@ -99,12 +99,20 @@ __device__ __forceinline__ void nbody_store(const NbodyParams& p, int64_t i, con
 #pragma unroll
     for (int r = 0; r < NR; r++) p.out[r * p.m + i] = pf * (acc[2 * r] - acc[2 * r + 1]);
   } else if (KIND == NB_VECTOR) {
-    p.out[3 * i] = pf * acc[3];
-    p.out[3 * i + 1] = -(pf * acc[2]);
-    p.out[3 * i + 2] = pf * (acc[0] - acc[1]);
+#pragma unroll
+    for (int r = 0; r < NR; r++) {
+      const int64_t t = r * p.m + i;
+      p.out[3 * t] = pf * acc[4 * r + 3];
+      p.out[3 * t + 1] = -(pf * acc[4 * r + 2]);
+      p.out[3 * t + 2] = pf * (acc[4 * r] - acc[4 * r + 1]);
+    }
   } else if (KIND == NB_VECPOT) {
-    p.out[2 * i] = pf * acc[0];
-    p.out[2 * i + 1] = pf * acc[1];
+#pragma unroll
+    for (int r = 0; r < NR; r++) {
+      const int64_t t = r * p.m + i;
+      p.out[2 * t] = pf * acc[2 * r];
+      p.out[2 * t + 1] = pf * acc[2 * r + 1];
+    }
   } else if (KIND == NB_FILM_TO_FILM) {
 #pragma unroll
     for (int r = 0; r < NR; r++) p.out[r * p.m + i] = pf * acc[r];
@@ -198,12 +206,6 @@ __global__ void __launch_bounds__(256) nbody_kernel(NbodyParams p, ShiftTable st
         if (KIND == NB_KERNEL) {
 #pragma unroll
           for (int r = 0; r < NR; r++) spay[r][tid] = p.J ? w * p.J[js * p.ldv + p.rhs0 + r] : w;
-        } else if (KIND == NB_FILM_TO_FILM || KIND == NB_Z) {
-#pragma unroll
-          for (int r = 0; r < NR; r++) {
-            spay[2 * r][tid] = w * p.J[(r * p.n + js) * 2];
-            spay[2 * r + 1][tid] = w * p.J[(r * p.n + js) * 2 + 1];
-          }
         } else if (KIND == NB_BOUNDARY) {
 #pragma unroll
           for (int r = 0; r < NR; r++) {
@@ -211,9 +213,12 @@ __global__ void __launch_bounds__(256) nbody_kernel(NbodyParams p, ShiftTable st
             spay[2 * r][tid] = wr * p.J[2 * js];
             spay[2 * r + 1][tid] = wr * p.J[2 * js + 1];
           }
-        } else {
-          spay[0][tid] = w * p.J[2 * js];
-          spay[1][tid] = w * p.J[2 * js + 1];
+        } else {  // NB_FILM_TO_FILM, NB_Z, NB_VECTOR, NB_VECPOT: J [NR, n, 2]
+#pragma unroll
+          for (int r = 0; r < NR; r++) {
+            spay[2 * r][tid] = w * p.J[(r * p.n + js) * 2];
+            spay[2 * r + 1][tid] = w * p.J[(r * p.n + js) * 2 + 1];
+          }
         }
       }
     }
@@ -244,10 +249,13 @@ __global__ void __launch_bounds__(256) nbody_kernel(NbodyParams p, ShiftTable st
           } else if (KIND == NB_FILM_TO_FILM) {
             r2 += p.dz2;
           }
-          if (KIND == NB_VECPOT) {
+          if (KIND == NB_VECPOT) {  // one r^-1 per pair for every set of the pass
             const double inv = inv_r1(r2);
-            acc[k][0] = fma(pay[0], inv, acc[k][0]);
-            acc[k][1] = fma(pay[1], inv, acc[k][1]);
+#pragma unroll
+            for (int r = 0; r < NR; r++) {
+              acc[k][2 * r] = fma(pay[2 * r], inv, acc[k][2 * r]);
+              acc[k][2 * r + 1] = fma(pay[2 * r + 1], inv, acc[k][2 * r + 1]);
+            }
           } else {
             double k3 = inv_r3(r2);
             if (KIND == NB_KERNEL) {
@@ -269,11 +277,14 @@ __global__ void __launch_bounds__(256) nbody_kernel(NbodyParams p, ShiftTable st
                 acc[k][2 * r + 1] = fma(k3 * pay[2 * r + 1], dx, acc[k][2 * r + 1]);  // Jy_dx
               }
             } else {                                        // NB_VECTOR
-              const double px = k3 * pay[0], py = k3 * pay[1];
-              acc[k][0] = fma(px, dy, acc[k][0]);   // Jx_dy
-              acc[k][1] = fma(py, dx, acc[k][1]);   // Jy_dx
-              acc[k][2] = fma(px, dzv, acc[k][2]);  // Jx_dz
-              acc[k][3] = fma(py, dzv, acc[k][3]);  // Jy_dz
+#pragma unroll
+              for (int r = 0; r < NR; r++) {
+                const double px = k3 * pay[2 * r], py = k3 * pay[2 * r + 1];
+                acc[k][4 * r] = fma(px, dy, acc[k][4 * r]);           // Jx_dy
+                acc[k][4 * r + 1] = fma(py, dx, acc[k][4 * r + 1]);   // Jy_dx
+                acc[k][4 * r + 2] = fma(px, dzv, acc[k][4 * r + 2]);  // Jx_dz
+                acc[k][4 * r + 3] = fma(py, dzv, acc[k][4 * r + 3]);  // Jy_dz
+              }
             }
           }
         }
@@ -300,7 +311,7 @@ __global__ void __launch_bounds__(256) nbody_kernel(NbodyParams p, ShiftTable st
 template <int KIND, int NR>
 __global__ void __launch_bounds__(128) nbody_reduce_kernel(NbodyParams p, int nsplit) {
   constexpr int NACC = Traits<KIND, NR>::nacc;
-  constexpr int TPB = 128 / NACC;  // targets per CTA (NACC in {1, 2, 4, 8, 16})
+  constexpr int TPB = 128 / NACC;  // targets per CTA (NACC in {1, 2, 4, 8, 16, 32})
   static_assert(128 % NACC == 0, "accumulator count must divide the CTA size");
   __shared__ double tot[TPB][NACC + 1];
   const int a = threadIdx.x % NACC, t = threadIdx.x / NACC;
@@ -332,10 +343,10 @@ static int launch_nbody(NbodyParams p, cudaStream_t s, ShiftTable st = {}) {
   const int64_t ctas_x = ceil_div(p.m, 256 * TPT);
   // One balanced wave: every CTA does the same amount of work, so the source range is split until the
   // grid just fills the resident-CTA capacity of the device (a CTA keeps at least one source tile).
-  // NB_Z passes of several sets split as the single-set pass does, whatever their own occupancy: the
-  // split fixes the summation order, so every set of a multi-set call has the bits of a one-set call.
-  // NB_COUPLING_T passes split as the one-set NB_COUPLING pass does, for the same reason.
-  constexpr int CAP_NR = (KIND == NB_Z || KIND == NB_COUPLING_T) ? 1 : NR;
+  // NB_Z, NB_VECTOR and NB_VECPOT passes of several sets split as the single-set pass does, whatever their own
+  // occupancy: the split fixes the summation order, so every set of a multi-set call has the bits of a one-set
+  // call.  NB_COUPLING_T passes split as the one-set NB_COUPLING pass does, for the same reason.
+  constexpr int CAP_NR = (KIND == NB_Z || KIND == NB_VECTOR || KIND == NB_VECPOT || KIND == NB_COUPLING_T) ? 1 : NR;
   constexpr int CAP_KIND = KIND == NB_COUPLING_T ? NB_COUPLING : KIND;
   static int capacity = 0;  // per instantiation; all devices of a node are identical
   if (capacity == 0) {
@@ -707,8 +718,18 @@ extern "C" int scb_biot_savart(int kind, int64_t m, const double* tgt, int64_t n
         else if (nsets - k >= 2) { rc = launch_nbody<NB_Z, 2>(p, s); step = 2; }
         else rc = launch_nbody<NB_Z, 1>(p, s);
         break;
-      case SCB_BS_VECTOR: rc = launch_nbody<NB_VECTOR, 1>(p, s); break;
-      case SCB_BS_VECTOR_POTENTIAL: rc = launch_nbody<NB_VECPOT, 1>(p, s); break;
+      case SCB_BS_VECTOR:  // one r^-3 per pair for the sets of a pass
+        if (nsets - k >= 8) { rc = launch_nbody<NB_VECTOR, 8>(p, s); step = 8; }
+        else if (nsets - k >= 4) { rc = launch_nbody<NB_VECTOR, 4>(p, s); step = 4; }
+        else if (nsets - k >= 2) { rc = launch_nbody<NB_VECTOR, 2>(p, s); step = 2; }
+        else rc = launch_nbody<NB_VECTOR, 1>(p, s);
+        break;
+      case SCB_BS_VECTOR_POTENTIAL:  // one r^-1 per pair for the sets of a pass
+        if (nsets - k >= 8) { rc = launch_nbody<NB_VECPOT, 8>(p, s); step = 8; }
+        else if (nsets - k >= 4) { rc = launch_nbody<NB_VECPOT, 4>(p, s); step = 4; }
+        else if (nsets - k >= 2) { rc = launch_nbody<NB_VECPOT, 2>(p, s); step = 2; }
+        else rc = launch_nbody<NB_VECPOT, 1>(p, s);
+        break;
       default: set_error("scb_biot_savart: unknown kind %d", kind); return SCB_ERR_INVALID;
     }
     if (rc) return rc;

@@ -709,29 +709,36 @@ class Solution:
 
 
 class _FilmBatch(NamedTuple):
-    """One film's share of a staged ``field_at_position_batch``."""
+    """One film's share of a staged batch evaluation."""
 
     name: str
-    src: np.ndarray                # (n, 3) vertices and layer height, meters
-    areas: np.ndarray              # (n,) vertex areas, square meters
-    J: Any                         # pinned (B, n, 2) current densities, A / m
+    src: np.ndarray                # (n, 3) vertices and layer height (meters; length units for the vector potential)
+    areas: np.ndarray              # (n,) vertex areas (square meters; squared length units)
+    J: Any                         # pinned (B, n, 2) current densities (A / m; current / length units)
     out_idx: Optional[np.ndarray]  # positions evaluated by the pair sum (None: all of them)
     in_idx: Optional[np.ndarray]   # positions inside the film, in its plane
-    in_field: Optional[np.ndarray]  # (B, len(in_idx)) interpolated self field there, tesla
+    in_field: Optional[np.ndarray]  # (B, len(in_idx)) interpolated self field (Bz) there, tesla
 
 
 class _FieldBatchStage(NamedTuple):
-    """Host side of ``field_at_position_batch``: checked inputs and staged arrays, no device work."""
+    """Host side of the batch evaluators: checked inputs and staged arrays, no device work."""
 
     B: int
     m: int
-    targets: Any                   # pinned (m, 3) evaluation points, meters
+    targets: Any                   # pinned (m, 3) evaluation points (meters; length units for the vector potential)
     films: List[_FilmBatch]
-    to_field_units: float          # tesla -> field_units
-    to_units: float                # field_units -> units
+    kind: int                      # scb_biot_savart kind: 1 Bz, 2 (Bx, By, Bz), 3 vector potential
+    prefactor: float
+    chunked: bool                  # targets in _EVAL_CHUNK launches (biot_savart_2d) or all in one launch
+    factors: Tuple[float, ...]     # unit factors applied to every film's result in turn (tesla -> ... -> units)
     units: str
-    applied: np.ndarray            # (k, m) distinct applied-field rows, in units
-    applied_row: np.ndarray        # (B,) row of ``applied`` of every entry
+    applied: Optional[np.ndarray]  # field_at_position: (k, m) distinct applied-field rows, in units
+    applied_row: Optional[np.ndarray]  # (B,) row of ``applied`` of every entry
+
+
+# B * points * components of one film's device result: bounds that buffer to 512 MiB by evaluating the entries in
+# groups (a group of sets changes no bit of a pair sum, a chunk of targets would)
+_BATCH_RESULT_ELEMS = 1 << 26
 
 
 def _interp_batch(mesh, rows: Sequence[Optional[np.ndarray]], xy: np.ndarray) -> np.ndarray:
@@ -749,7 +756,11 @@ def _interp_batch(mesh, rows: Sequence[Optional[np.ndarray]], xy: np.ndarray) ->
     return out
 
 
-def _stage_field_batch(solutions, positions, zs, interp_method: str, units: Optional[str]) -> _FieldBatchStage:
+def _stage_field_batch(solutions, positions, zs, interp_method: str, units: Optional[str], what: str = "field",
+                       vector: bool = False) -> _FieldBatchStage:
+    """``what``: "field" (field_at_position), "screening" (screening_field_at_position, Bz or with ``vector`` the
+    vector field) or "vector_potential" (vector_potential_at_position).  The operands are those of the per-solution
+    methods: meters and A / m for the fields (biot_savart_2d), length and current units for the vector potential."""
     import torch
 
     solutions = list(solutions)
@@ -758,8 +769,9 @@ def _stage_field_batch(solutions, positions, zs, interp_method: str, units: Opti
             raise TypeError(f"solutions[{b}] is a {type(sol).__name__}, not a Solution.")
     positions, zs = _normalize_positions(positions, zs, np.float64)
     B, m = len(solutions), len(positions)
+    kind = 3 if what == "vector_potential" else (2 if vector else 1)
     if B == 0:
-        return _FieldBatchStage(0, m, None, [], 1.0, 1.0, units, np.zeros((0, m)), np.zeros(0, dtype=np.int64))
+        return _FieldBatchStage(0, m, None, [], kind, 1.0, True, (), units, None, None)
     first = solutions[0]
     device = first.device
     film_names = list(device.films)
@@ -784,14 +796,28 @@ def _stage_field_batch(solutions, positions, zs, interp_method: str, units: Opti
             z0, z0_first = d.layers[d.films[name].layer].z0, device.layers[device.films[name].layer].z0
             if z0 != z0_first:
                 raise ValueError(f"solutions[{b}] has film {name!r} at z0 = {z0}, solutions[0] at z0 = {z0_first}.")
-    in_plane = [np.all(zs == device.layers[film.layer].z0) for film in device.films.values()]
-    if interp_method != "linear" and any(in_plane):  # (as interp_field raises it)
-        raise NotImplementedError("Only linear interpolation is available.")
-
     field_units, current_units, length_units = first.field_units, first.current_units, device.length_units
-    units = units or field_units
-    to_meter = _u.conversion_factor(length_units, "m")
-    to_amp_per_meter = _u.conversion_factor(f"({current_units}) / ({length_units})", "A / m")
+    if what == "vector_potential":
+        for name, film in device.films.items():  # (as vector_potential_at_position raises it)
+            if np.all(zs - device.layers[film.layer].z0 == 0) and film.contains_points(positions).all():
+                raise ValueError(f"Cannot evaluate vector potential inside the film ({name!r}).")
+        in_plane = [False] * len(film_names)
+        units = units or f"({field_units}) * ({length_units})"
+        to_meter = to_amp_per_meter = 1.0  # (multiplying by one is exact: the operands of the per-solution call)
+        prefactor = (_u.MU_0 / (4 * np.pi) * _u.conversion_factor(current_units, "A")
+                     * _u.conversion_factor("T * m", units))
+        factors: Tuple[float, ...] = ()
+    else:
+        in_plane = [np.all(zs == device.layers[film.layer].z0) for film in device.films.values()]
+        if interp_method != "linear" and any(in_plane):  # (as interp_field raises it)
+            raise NotImplementedError("Only linear interpolation is available.")
+        units = units or field_units
+        to_meter = _u.conversion_factor(length_units, "m")
+        to_amp_per_meter = _u.conversion_factor(f"({current_units}) / ({length_units})", "A / m")
+        prefactor = _MU0_BIOT_SAVART / (4 * np.pi)
+        # field_at_position converts the screening fields to field_units, then everything to units
+        factors = ((_field_factor("tesla", field_units), _field_factor(field_units, units)) if what == "field"
+                   else (_field_factor("tesla", units),))
     # (the same host arithmetic as biot_savart_2d, so the device sees the same operands)
     targets = torch.empty((m, 3), dtype=torch.float64, pin_memory=True)
     ev = targets.numpy()
@@ -822,6 +848,9 @@ def _stage_field_batch(solutions, positions, zs, interp_method: str, units: Opti
         for b, sol in enumerate(solutions):
             Jh[b] = np.atleast_2d(sol.film_solutions[name].current_density) * to_amp_per_meter
         films.append(_FilmBatch(name, src, areas, J, out_idx, in_idx, in_field))
+    if what != "field":
+        return _FieldBatchStage(B, m, targets, films, kind, prefactor, what != "vector_potential", factors, units,
+                                None, None)
 
     # applied field (field_at_position): interpolated from the solutions at in-plane points inside a film, the
     # applied-field function elsewhere -- evaluated once per distinct function object
@@ -859,77 +888,113 @@ def _stage_field_batch(solutions, positions, zs, interp_method: str, units: Opti
             for b in range(B):
                 per_entry[b, mask] = rows[applied_row[b]]
         applied, applied_row = per_entry, np.arange(B)
-    to_units = _field_factor(field_units, units)
+    to_units = factors[1]
     if to_units != 1.0:
         applied = applied * to_units
-    return _FieldBatchStage(B, m, targets, films, _field_factor("tesla", field_units), to_units, units,
-                            applied, applied_row)
+    return _FieldBatchStage(B, m, targets, films, kind, prefactor, True, factors, units, applied, applied_row)
 
 
 def _evaluate_field_batch(stage: _FieldBatchStage, return_sum: bool):
-    """Device side of ``field_at_position_batch``: one multi-set pair sum per film and chunk of targets, the unit
-    factors and the sum over films on the device, one copy of every result to the host."""
+    """Device side of the batch evaluators: for every group of entries, one multi-set pair sum per film (and chunk
+    of targets), the unit factors and the sum over films on the device, one copy of every group's result to the
+    host.  Returns (B, m) arrays (Bz) or (B, m, 3) arrays (vector field, vector potential with a zero z column)."""
     import torch
 
     L = _lib.lib()
     B, m = stage.B, stage.m
+    tail = () if stage.kind == 1 else (3,)
+    ncomp = 3 if stage.kind == 2 else (2 if stage.kind == 3 else 1)  # components the pair sum writes
+    group = max(1, min(B, _BATCH_RESULT_ELEMS // max(m * (1 if stage.kind == 1 else 3), 1)))
     dev = torch.device(f"cuda:{torch.cuda.current_device()}")
     with torch.cuda.device(dev):
         targets = stage.targets.to(dev, non_blocking=True)
-        total, fields = None, {}
+        per_film = []  # (sources, areas, targets of the pair sum, their indices or None) of every film
         for f in stage.films:
-            src, areas, J = (torch.as_tensor(a).to(dev, non_blocking=True) for a in (f.src, f.areas, f.J))
-            field = torch.empty((B, m), dtype=torch.float64, device=dev)
-            if f.out_idx is None:
-                tgt = targets
-            else:
-                out_idx = torch.as_tensor(f.out_idx).to(dev)
-                tgt = targets.index_select(0, out_idx)
-                field[:, torch.as_tensor(f.in_idx).to(dev)] = torch.as_tensor(f.in_field).to(dev)
-            # the chunks of biot_savart_2d: the source split of the pair sum, hence every bit of it, depends on
-            # the number of targets of a launch
-            mf = int(tgt.shape[0])
-            chunk = mf if mf <= _EVAL_CHUNK else _EVAL_CHUNK
-            for lo in range(0, mf, max(chunk, 1)):
-                hi = min(mf, lo + chunk)
-                direct = f.out_idx is None and hi - lo == m
-                out = field if direct else torch.empty((B, hi - lo), dtype=torch.float64, device=dev)
-                _lib.check(L.scb_biot_savart(1, hi - lo, _lib.ptr(tgt[lo:hi]), int(src.shape[0]), _lib.ptr(src),
-                                             _lib.ptr(areas), _lib.ptr(J), 0.0, _MU0_BIOT_SAVART / (4 * np.pi), B,
-                                             _lib.ptr(out), _lib.stream_ptr()))
-                if f.out_idx is not None:
-                    field[:, out_idx[lo:hi]] = out
-                elif not direct:
-                    field[:, lo:hi] = out
-            # tesla -> field_units -> units, then films in device order: the operations of field_at_position
-            if stage.to_field_units != 1.0:
-                field.mul_(stage.to_field_units)
-            if stage.to_units != 1.0:
-                field.mul_(stage.to_units)
-            if not return_sum:
-                fields[f.name] = field
-            elif total is None:
-                total = field
-            else:
-                total.add_(field)
-        results = fields
-        if return_sum:
-            applied = torch.as_tensor(stage.applied).to(dev).index_select(0, torch.as_tensor(stage.applied_row).to(dev))
-            if total is None:
-                total = applied
-            else:
-                total.add_(applied)
-            results = {"total": total}
-        host = {}
-        for key, t in results.items():
-            host[key] = torch.empty((B, m), dtype=torch.float64, pin_memory=True)
-            host[key].copy_(t, non_blocking=True)
+            src, areas = (torch.as_tensor(a).to(dev, non_blocking=True) for a in (f.src, f.areas))
+            out_idx = None if f.out_idx is None else torch.as_tensor(f.out_idx).to(dev)
+            per_film.append((src, areas, targets if out_idx is None else targets.index_select(0, out_idx), out_idx))
+        applied = None
+        if return_sum and stage.applied is not None:
+            applied = torch.as_tensor(stage.applied).to(dev)
+            applied_row = torch.as_tensor(stage.applied_row).to(dev)
+        keys = ["total"] if return_sum else [f.name for f in stage.films]
+        host = {key: torch.empty((B, m) + tail, dtype=torch.float64, pin_memory=True) for key in keys}
+        for g0 in range(0, B, group):
+            g1 = min(B, g0 + group)
+            G = g1 - g0
+            total, fields = None, {}
+            for f, (src, areas, tgt, out_idx) in zip(stage.films, per_film):
+                J = f.J[g0:g1].to(dev, non_blocking=True)
+                field = torch.empty((G, m) + tail, dtype=torch.float64, device=dev)
+                if stage.kind == 3:
+                    field[..., 2] = 0.0
+                if f.in_idx is not None:
+                    in_idx = torch.as_tensor(f.in_idx).to(dev)
+                    in_field = torch.as_tensor(f.in_field[g0:g1]).to(dev)
+                    if stage.kind == 1:
+                        field[:, in_idx] = in_field
+                    else:  # (the in-plane self field has a z component only)
+                        block = torch.zeros((G, len(f.in_idx), 3), dtype=torch.float64, device=dev)
+                        block[..., 2] = in_field
+                        field[:, in_idx] = block
+                # the chunks of biot_savart_2d: the source split of the pair sum, hence every bit of it, depends on
+                # the number of targets of a launch (vector_potential_at_position: all targets in one launch)
+                mf = int(tgt.shape[0])
+                chunk = mf if (mf <= _EVAL_CHUNK or not stage.chunked) else _EVAL_CHUNK
+                for lo in range(0, mf, max(chunk, 1)):
+                    hi = min(mf, lo + chunk)
+                    direct = out_idx is None and hi - lo == m and stage.kind != 3
+                    out = field if direct else torch.empty((G, hi - lo) + (() if ncomp == 1 else (ncomp,)),
+                                                           dtype=torch.float64, device=dev)
+                    _lib.check(L.scb_biot_savart(stage.kind, hi - lo, _lib.ptr(tgt[lo:hi]), int(src.shape[0]),
+                                                 _lib.ptr(src), _lib.ptr(areas), _lib.ptr(J), 0.0, stage.prefactor,
+                                                 G, _lib.ptr(out), _lib.stream_ptr()))
+                    if direct:
+                        continue
+                    rows = slice(lo, hi) if out_idx is None else out_idx[lo:hi]
+                    if stage.kind == 3:
+                        field[:, rows, :2] = out
+                    else:
+                        field[:, rows] = out
+                # unit factors, then films in device order: the operations of the per-solution methods
+                for factor in stage.factors:
+                    if factor != 1.0:
+                        field.mul_(factor)
+                if not return_sum:
+                    fields[f.name] = field
+                elif total is None:
+                    total = field
+                else:
+                    total.add_(field)
+            if return_sum:
+                if applied is not None:
+                    rows_g = applied.index_select(0, applied_row[g0:g1])
+                    if total is None:
+                        total = rows_g
+                    else:
+                        total.add_(rows_g)
+                elif total is None:
+                    total = torch.zeros((G, m) + tail, dtype=torch.float64, device=dev)
+                fields = {"total": total}
+            for key, t in fields.items():
+                host[key][g0:g1].copy_(t, non_blocking=True)
         torch.cuda.current_stream(dev).synchronize()
     if return_sum:
         return host["total"].numpy()
     out = {key: t.numpy() for key, t in host.items()}
-    out["applied_field"] = stage.applied[stage.applied_row]
+    if stage.applied is not None:
+        out["applied_field"] = stage.applied[stage.applied_row]
     return out
+
+
+def _batch_result(stage: _FieldBatchStage, return_sum: bool, with_units: bool, tail: tuple = ()):
+    value = _evaluate_field_batch(stage, return_sum) if stage.B else (np.empty((0, stage.m) + tail) if return_sum
+                                                                      else {})
+    if not with_units or (stage.B == 0 and stage.units is None):
+        return value
+    if return_sum:
+        return _u.Quantity(value, stage.units)
+    return {key: _u.Quantity(v, stage.units) for key, v in value.items()}
 
 
 def field_at_position_batch(solutions: Sequence["Solution"], positions, *, zs=None, interp_method: str = "linear",
@@ -945,15 +1010,36 @@ def field_at_position_batch(solutions: Sequence["Solution"], positions, *, zs=No
     units and the current units; each must hold every film.  Applied-field functions are evaluated once per
     distinct function object."""
     stage = _stage_field_batch(solutions, positions, zs, interp_method, units)
-    if stage.B == 0:
-        value = np.empty((0, stage.m)) if return_sum else {}
-    else:
-        value = _evaluate_field_batch(stage, return_sum)
-    if not with_units or (stage.B == 0 and units is None):
-        return value
-    if return_sum:
-        return _u.Quantity(value, stage.units)
-    return {key: _u.Quantity(v, stage.units) for key, v in value.items()}
+    return _batch_result(stage, return_sum, with_units)
+
+
+def screening_field_at_position_batch(solutions: Sequence["Solution"], positions, *, zs=None, vector: bool = False,
+                                      interp_method: str = "linear", units: Optional[str] = None,
+                                      with_units: bool = True, return_sum: bool = True):
+    """``Solution.screening_field_at_position`` of B solutions of one device at the same positions, in one pass:
+    row ``b`` is ``solutions[b].screening_field_at_position(positions, zs=zs, vector=vector,
+    interp_method=interp_method, units=units, with_units=False, return_sum=return_sum)``.
+
+    Returns a ``(B, m)`` array, ``(B, m, 3)`` with ``vector=True`` (a ``Quantity`` with ``with_units``), or with
+    ``return_sum=False`` a dict of such arrays, one per film.  Every film's field at the points off its plane is one
+    pair sum over all B current densities (one r^-3 per pair serves up to 8 entries), with the bits of the
+    per-solution call; at in-plane points inside a film the film's self field is interpolated, as there.  The
+    solutions must meet the conditions of ``field_at_position_batch``."""
+    stage = _stage_field_batch(solutions, positions, zs, interp_method, units, what="screening", vector=vector)
+    return _batch_result(stage, return_sum, with_units, (3,) if vector else ())
+
+
+def vector_potential_at_position_batch(solutions: Sequence["Solution"], positions, *, zs=None,
+                                       units: Optional[str] = None, with_units: bool = True, return_sum: bool = True):
+    """``Solution.vector_potential_at_position`` of B solutions of one device at the same positions, in one pass: a
+    ``(B, m, 3)`` array (zero z column) whose row ``b`` is ``solutions[b].vector_potential_at_position(positions,
+    zs=zs, units=units, with_units=False, return_sum=return_sum)``, bit for bit (a ``Quantity`` with
+    ``with_units``), or with ``return_sum=False`` a dict of such arrays, one per film.  One pair sum per film serves
+    all B current densities (one r^-1 per pair for up to 8 entries).  Raises the ``ValueError`` of the per-solution
+    method when every position lies inside a film in its plane, before any device work.  The solutions must meet
+    the conditions of ``field_at_position_batch``."""
+    stage = _stage_field_batch(solutions, positions, zs, "linear", units, what="vector_potential")
+    return _batch_result(stage, return_sum, with_units, (3,))
 
 
 # interpolated values per chunk of targets (B * points * components): bounds the device output buffer to 512 MiB
